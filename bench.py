@@ -8,7 +8,7 @@ BASELINE.json's target is quoted on): MiniZephyr 1000x3000 grid, dx=dz=10 m, ran
 velocity, 512 sources / 512 receivers, one frequency per GPU (weak scaling: N GPUs run the first
 N of linspace(2,9,8) Hz).  `value` = source-frequency wavefields per second, whole job.
 
-    python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--nx --nz --nsrc]
+    python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--nx --nz --nsrc] [--dump-outputs DIR]
 """
 import argparse
 import json
@@ -29,6 +29,7 @@ import numpy as np  # noqa: E402
 METRIC = 'source-frequency wavefields/sec'
 UNIT = 'wavefields/s'
 NOMINAL_FP64_TFLOPS = 148 * 128 * 1.965e9 / 1e12      # 148 SMs x 128 flop/clk x max SM clock
+DUMP_BYTES = 64 << 20                                 # --dump-outputs: at most this much per rank
 
 
 def layered_model(nx, nz, rng, lo=1500., hi=4500., tmin=5, tmax=50):
@@ -187,6 +188,25 @@ def c4_config(nfreq=16, nsrc=256, nrec=256, nx=500, nz=1500, npml=20):
     sc = {'nx': nx, 'nz': nz, 'dx': dx, 'dz': dx, 'c': c, 'rho': 1., 'nPML': npml, 'freqs': list(np.linspace(2., 12., 16)[:nfreq]),
           'geom': {'src': np.stack([xs, np.full(nsrc, zs)], 1), 'rec': np.stack([xr, np.full(nrec, zs + dx)], 1), 'mode': 'fixed'}}
     return sc, c * (1. - 0.1 * blob)
+
+
+def dump_outputs(dirname, outputs, rank, world):
+    """--dump-outputs: write what the timed path returned in its last step as DIR/<name>.npy, so that two builds can be
+    compared output for output.  `outputs` maps name -> (device tensor, byte budget).  Complex tensors are stored as
+    real arrays with a trailing (re, im) axis: float64, or float32 for complex64.  A tensor larger than its budget is
+    cut to a fixed sample of its rows (first axis; seed 0, sorted), the same rows in every run with the same arguments.
+    With several ranks each writes its own frequencies as <name>.rank<r>.npy."""
+    import torch
+    assert sum(b for _, b in outputs.values()) <= DUMP_BYTES
+    os.makedirs(dirname, exist_ok=True)
+    for name, (t, budget) in outputs.items():
+        if t.is_complex():
+            t = torch.view_as_real(t)
+        row_bytes = t[0].numel() * t.element_size()
+        if t.numel() * t.element_size() > budget:
+            keep = np.sort(np.random.default_rng(0).choice(t.shape[0], budget // row_bytes, replace=False))
+            t = t[torch.from_numpy(keep).to(t.device)]
+        np.save(os.path.join(dirname, name + ('' if world == 1 else '.rank%d' % rank) + '.npy'), t.cpu().numpy())
 
 
 def workload_config(a, nfreq):
@@ -365,6 +385,8 @@ def run_c4(a, torch, zb, _lib, parallel, rank, world, dev, local):
     ms_per_step = float(tt.item()) / a.steps
     value = 2 * F * S / (ms_per_step * 1e-3)             # forward + adjoint wavefields
     assert bool(torch.isfinite(red).all())
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {'gradient': (red[:-1], DUMP_BYTES - (1 << 20)), 'misfit': (red[-1:], 1 << 20)}, rank, world)
     # end to end: host model in, host gradient + misfit out
     c_host = torch.from_numpy(np.ascontiguousarray(sc['c'], dtype=np.complex128)).pin_memory()
     e2e = None
@@ -588,7 +610,13 @@ def main():
     ap.add_argument('--opt', action='append', default=[], help='library option key=value (hz_set_option), e.g. gj_pdl=1')
     ap.add_argument('--workers', type=int, default=0, help='c2/c4: host threads (frequencies in flight) per GPU for factorisation and sweeps (0: library default 4)')
     ap.add_argument('--twist', type=int, default=-1, help='block row where the elimination chains meet (-1: nz/2 (default policy), -2: source depth)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='after the timed steps, write what the last step returned as DIR/<name>.npy '
+                    '(c3: receiver data + a fixed row sample of the wavefield panel; c2: receiver data; c4: gradient + misfit)')
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
+    if a.dump_outputs and (a.impl == 'reference' or a.config == 'c5'):
+        ap.error('--dump-outputs covers the c2, c3 and c4 GPU paths')
     if a.impl == 'reference':
         return run_reference(a)
 
@@ -641,6 +669,7 @@ def main():
         torch.cuda.synchronize()
 
     tms = {'assemble': 0.0, 'factor': 0.0, 'solve': 0.0, 'extract': 0.0}
+    last = {}
 
     def step(record=False):
         if len(mine) > 1:
@@ -653,6 +682,7 @@ def main():
             ev[1].record()
             dd = pr.dpred_device()        # each worker factors and sweeps its own frequencies: phases of different frequencies overlap
             ev[2].record()
+            last['data'] = dd
             if record:
                 ev[2].synchronize()
                 tms['assemble'] += ev[0].elapsed_time(ev[1])
@@ -706,6 +736,12 @@ def main():
     ms_per_step = ms / a.steps
     value = nfreq * S / (ms_per_step * 1e-3)
     assert bool(torch.isfinite(torch.view_as_real(d)).all())
+    if a.dump_outputs:
+        if 'data' in last:                # several frequencies: the (R, S) data of each, the wavefield panels stay internal
+            out = {'data': (torch.stack([last['data'][i] for i in mine]), DUMP_BYTES)}
+        else:                             # receiver data and the (N, S) wavefield panel the last step solved for
+            out = {'data': (d, 16 << 20), 'wavefield': (X, DUMP_BYTES - (16 << 20))}
+        dump_outputs(a.dump_outputs, out, rank, world)
     fp32_peak = 148 * 128 * 2 * 1.965e9 / 1e12      # nominal FP32 FFMA peak (no measured figure in MEASURED_PEAKS.json)
 
     # ---- end to end through the reference-facing call: host model in, host data out ----------
