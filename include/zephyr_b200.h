@@ -43,6 +43,7 @@ enum {
 };
 enum { HZ_C128 = 0, HZ_C64 = 1 };
 enum { HZ_DISC_MINIZEPHYR = 0, HZ_DISC_EURUS = 1 };
+enum { HZ_OP_N = 0, HZ_OP_T = 1, HZ_OP_H = 2 };   /* which operator a solve inverts: A, A^T, A^H (conjugate transpose) */
 
 const char* hz_version(void);
 const char* hz_last_error(hz_handle_t h);
@@ -95,10 +96,17 @@ int hz_get_block_inverse(hz_handle_t h, int64_t iz, void* out_host);   /* (b x b
  * resid_host (optional): ||q - A x||_F / ||q||_F of the final solution.                          */
 int hz_solve(hz_handle_t h, void* X, int64_t S, double premul_re, double premul_im, int conjugate,
              int64_t z_first, int64_t z_last, int refine, double* resid_host);
+/* X <- conj(premul * op(A)^{-1} X), op = HZ_OP_N (== hz_solve), HZ_OP_T (A^T) or HZ_OP_H (A^H), from the same factors:
+ * the Schur complements of A^T are the transposes of those of A, so the sweeps apply the stored block inverses as
+ * S_i^{-T} / S_i^{-H} with the transposed (conjugated) stencil -- scipy's SuperLU.solve(rhs, trans='N'|'T'|'H').  Other
+ * arguments, the accuracy probe (the first solve after hz_factor probes, whatever its op) and the refinement use the
+ * op(A) residual and otherwise behave as in hz_solve.  Bad op -> HZ_EINVAL; T / H on a complex64 handle -> HZ_ENOTIMPL. */
+int hz_solve_op(hz_handle_t h, int op, void* X, int64_t S, double premul_re, double premul_im, int conjugate,
+                int64_t z_first, int64_t z_last, int refine, double* resid_host);
 
 /* Accuracy probe.  The reference's SuperLU pivots; the block elimination here does not pivot across
- * 32-wide panels.  The first hz_solve (refine = 0) after every hz_factor therefore measures, in FP64,
- * the 9-point stencil residual ||q - A x|| / ||q|| of the first right-hand-side column and returns
+ * 32-wide panels.  The first hz_solve / hz_solve_op (refine = 0) after every hz_factor therefore measures, in FP64,
+ * the 9-point stencil residual ||q - op(A) x|| / ||q|| of the first right-hand-side column and returns
  * HZ_EACCURACY when it exceeds 1e-7 (complex128) / 1e-2 (complex64) instead of a silently inaccurate
  * wavefield.  hz_last_probe returns the last measured value (-1: none yet); option "probe_check" = 0
  * disables the probe.  With refine >= 1 the refinement loop's own residual takes its place.        */
@@ -219,6 +227,12 @@ int hz_cgemm_tf32(int64_t M, int64_t N, int64_t K, double alpha, const float* A_
 /* Test hook for the DMMA contraction: C = beta*C + alpha*A*B (row-major complex128).            */
 int hz_zgemm(int64_t M, int64_t N, int64_t K, double alpha, const void* A, int64_t lda, const void* B,
              int64_t ldb, int beta, void* C, int64_t ldc, int tile, void* stream);
+/* ... with op(A): C = beta*C + alpha*op(A)*B, opA = HZ_OP_N (A is M x K), HZ_OP_T or HZ_OP_H (A is K x M, applied
+ * transposed / conjugate-transposed); tile: -1 = the host's pick for (M, N), 0..6 = candidate tiling 64x64, 56x64,
+ * 48x64, 40x64, 32x64, 32x32, 16x32; gemm_3m: 0 four, 1 three real products per complex product -- every kernel
+ * instance the substitution sweeps can run.                                                     */
+int hz_zgemm_op(int64_t M, int64_t N, int64_t K, double alpha, const void* A, int64_t lda, int opA, const void* B,
+                int64_t ldb, int beta, void* C, int64_t ldc, int tile, int gemm_3m, void* stream);
 
 #ifdef __cplusplus
 }

@@ -15,6 +15,7 @@ LIB_PATH = os.path.join(HERE, 'libzephyr_b200.so')
 HZ_OK, HZ_EINVAL, HZ_EDIM, HZ_ENOMEM, HZ_ECUDA, HZ_ESINGULAR, HZ_ESTATE, HZ_ENOTIMPL, HZ_EACCURACY = range(9)
 HZ_C128, HZ_C64 = 0, 1
 HZ_DISC_MINIZEPHYR, HZ_DISC_EURUS = 0, 1
+HZ_OP_N, HZ_OP_T, HZ_OP_H = 0, 1, 2
 
 _vp, _i64, _i32, _f64, _int = C.c_void_p, C.c_int64, C.c_int32, C.c_double, C.c_int
 
@@ -35,6 +36,7 @@ SIGNATURES = {
     'hz_factor_bytes': (_int, [_vp, C.POINTER(_i64)]),
     'hz_get_block_inverse': (_int, [_vp, _i64, _vp]),
     'hz_solve': (_int, [_vp, _vp, _i64, _f64, _f64, _int, _i64, _i64, _int, C.POINTER(_f64)]),
+    'hz_solve_op': (_int, [_vp, _int, _vp, _i64, _f64, _f64, _int, _i64, _i64, _int, C.POINTER(_f64)]),
     'hz_synchronize': (_int, [_vp]),
     'hz_last_probe': (_int, [_vp, C.POINTER(_f64)]),
     'hz_profile': (_int, [_vp, _int, C.POINTER(_f64)]),
@@ -58,6 +60,7 @@ SIGNATURES = {
     'hz_misfit_c64': (_int, [_vp, _vp, _i64, _f64, _vp, _vp, _vp]),
     'hz_cgemm_tf32': (_int, [_i64, _i64, _i64, _f64, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp, _int]),
     'hz_zgemm': (_int, [_i64, _i64, _i64, _f64, _vp, _i64, _vp, _i64, _int, _vp, _i64, _int, _vp]),
+    'hz_zgemm_op': (_int, [_i64, _i64, _i64, _f64, _vp, _i64, _int, _vp, _i64, _int, _vp, _i64, _int, _int, _vp]),
 }
 
 
@@ -115,6 +118,14 @@ def check(rc, handle=None):
     msg = get_lib().hz_last_error(handle)
     msg = msg.decode() if msg else 'zephyr_b200 error %d' % rc
     raise _EXC.get(rc, HzError)(msg)
+
+
+def trans_op(trans):
+    """``trans`` of scipy's ``SuperLU.solve`` ('N', 'T', 'H') -> HZ_OP_N / HZ_OP_T / HZ_OP_H."""
+    try:
+        return {'N': HZ_OP_N, 'T': HZ_OP_T, 'H': HZ_OP_H}[trans]
+    except (KeyError, TypeError):
+        raise ValueError("trans must be 'N', 'T' or 'H', not %r" % (trans,))
 
 
 def panel_fn(name, c64):

@@ -1060,8 +1060,10 @@ static void preload_kernel(K kfn) {
 }
 template <class TP>
 static void preload_panel_kernels() {
-    preload_kernel(couple_kernel<TP>); preload_kernel(residual_kernel<TP>); preload_kernel(gather_col_kernel<TP>);
-    preload_kernel(residual_col_kernel<TP>); preload_kernel(norm2_kernel<TP>); preload_kernel(axpy_kernel<TP>);
+    preload_kernel(couple_kernel<TP, 0>); preload_kernel(residual_kernel<TP, 0>); preload_kernel(gather_col_kernel<TP>);
+    preload_kernel(residual_col_kernel<TP, 0>); preload_kernel(norm2_kernel<TP>); preload_kernel(axpy_kernel<TP>);
+    preload_kernel(couple_kernel<TP, 1>); preload_kernel(residual_kernel<TP, 1>); preload_kernel(residual_col_kernel<TP, 1>);
+    preload_kernel(couple_kernel<TP, 2>); preload_kernel(residual_kernel<TP, 2>); preload_kernel(residual_col_kernel<TP, 2>);
     preload_kernel(finalize_kernel<TP>); preload_kernel(scatter_coo_kernel<TP>); preload_kernel(spmm_csr_kernel<TP>);
     preload_kernel(spmm_percol_kernel<TP>); preload_kernel(spmm_percol_t_kernel<TP>); preload_kernel(gradient_kernel<TP>);
     preload_kernel(misfit_kernel<TP>);
@@ -1090,7 +1092,9 @@ static void preload_factor_kernels() {
     preload_kernel(nearest_index_kernel); preload_kernel(kaiser_taps_kernel);
     preload_panel_kernels<cplx>();
     preload_panel_kernels<cplxf>();
-    zgemm_for_each_instance([](auto kfn) { preload_kernel(kfn); });
+    zgemm_for_each_instance<0>([](auto kfn) { preload_kernel(kfn); });
+    zgemm_for_each_instance<1>([](auto kfn) { preload_kernel(kfn); });
+    zgemm_for_each_instance<2>([](auto kfn) { preload_kernel(kfn); });
     // the service kernels request > 48 KB of dynamic shared memory: a per-device attribute as well
     cudaFuncSetAttribute(gj_inverter_service, cudaFuncAttributeMaxDynamicSharedMemorySize, GJ_SERVICE_SMEM);
     cudaFuncSetAttribute(gj_inverter_service2, cudaFuncAttributeMaxDynamicSharedMemorySize, GJ_SERVICE_SMEM);
@@ -1453,8 +1457,9 @@ int hz_get_block_inverse(hz_handle_t h, int64_t iz, void* out_host) {
 }
 
 // ---- substitution ----------------------------------------------------------------------------
+// op: HZ_OP_N / T / H -- which operator's off-diagonal blocks couple (complex64 panels: N only, hz_solve_op)
 template <class TP>
-static int launch_couple(hz_ctx* h, i64 i, TP* X, i64 S, TP* Y, int use_self, double lo, double hi, cudaStream_t st, int zero_self) {
+static int launch_couple(hz_ctx* h, i64 i, TP* X, i64 S, TP* Y, int use_self, double lo, double hi, cudaStream_t st, int zero_self, int op) {
     const int threads = S >= 128 ? 128 : (S >= 64 ? 64 : 32);
     dim3 grid((unsigned)((S + threads - 1) / threads), h->b, 1);
 #ifndef HZ_EMU
@@ -1474,14 +1479,14 @@ static int launch_couple(hz_ctx* h, i64 i, TP* X, i64 S, TP* Y, int use_self, do
         return HZ_OK;
     }
 #endif
-    auto kfn = couple_kernel<TP>;
+    auto kfn = op == HZ_OP_T ? couple_kernel<TP, 1> : (op == HZ_OP_H ? couple_kernel<TP, 2> : couple_kernel<TP, 0>);
     HZ_LAUNCH_EW(kfn, grid, dim3(threads), 0, st, (const cplx*)h->coef, h->nf, h->nx, h->nz, (int)i, X, S, Y, use_self, lo, hi);
     HZ_CHECK_LAUNCH(h);
     return HZ_OK;
 }
 
-// X_i <- beta X_i + alpha S_i^{-1} Y on the FP64 tensor pipe (complex128) ...
-static int launch_block_gemm(hz_ctx* h, i64 i, const cplx* Y, cplx* X, i64 S, double alpha, int beta, cudaStream_t st) {
+// X_i <- beta X_i + alpha op(S_i^{-1}) Y on the FP64 tensor pipe (complex128; op N, T or H: S_i(A^T) = S_i(A)^T) ...
+static int launch_block_gemm(hz_ctx* h, i64 i, const cplx* Y, cplx* X, i64 S, double alpha, int beta, cudaStream_t st, int op) {
     GemmParams p;
     p.A = h->Sinv + slot_of(h, i) * (i64)h->b * h->b; p.lda = h->b;
     p.B = Y; p.ldb = S;
@@ -1493,13 +1498,16 @@ static int launch_block_gemm(hz_ctx* h, i64 i, const cplx* Y, cplx* X, i64 S, do
     p.row_fs = h->N;
     bool armed;
     prof_begin(h, 0, st, armed);
-    zgemm_launch(p, st, h->num_sms, -1, (h->gemm_3m & 1) != 0);
+    const bool m3 = (h->gemm_3m & 1) != 0;
+    if (op == HZ_OP_T) zgemm_launch<1>(p, st, h->num_sms, -1, m3);
+    else if (op == HZ_OP_H) zgemm_launch<2>(p, st, h->num_sms, -1, m3);
+    else zgemm_launch<0>(p, st, h->num_sms, -1, m3);
     prof_end(h, 0, st, armed);
     HZ_CHECK_LAUNCH(h);
     return HZ_OK;
 }
-// ... or in FP32 on complex64 factors and panels
-static int launch_block_gemm(hz_ctx* h, i64 i, const cplxf* Y, cplxf* X, i64 S, double alpha, int beta, cudaStream_t st) {
+// ... or in FP32 on complex64 factors and panels (op N only: hz_solve_op rejects T / H for complex64 handles)
+static int launch_block_gemm(hz_ctx* h, i64 i, const cplxf* Y, cplxf* X, i64 S, double alpha, int beta, cudaStream_t st, int /*op*/) {
 #ifndef HZ_EMU
     if (h->tf32_active) {
         Tf32Params tp;
@@ -1562,9 +1570,11 @@ static int recompute_segment(hz_ctx* h, int chain, i64 j, cudaStream_t st) {
     return HZ_OK;
 }
 
-// X <- A^{-1} X (no premul / conjugation); zf/zl: first/last block row with non-zero rhs
+// X <- op(A)^{-1} X (no premul / conjugation); zf/zl: first/last block row with non-zero rhs.  The Schur complements of
+// A^T (A^H) are S_i^T (S_i^H) for both chains and the middle block, so every op runs the same two sweeps on the same
+// factors: op(S_i^{-1}) in the GEMMs and the op(A) stencil in the coupling.
 template <class TP>
-static int solve_inplace(hz_ctx* h, TP* X, i64 S, i64 zf, i64 zl) {
+static int solve_inplace(hz_ctx* h, TP* X, i64 S, i64 zf, i64 zl, int op) {
     const i64 nz = h->nz, mid = h->mid;
     const int k = h->store_used;
     if (zf < 0 || zf >= nz) zf = 0;
@@ -1584,15 +1594,15 @@ static int solve_inplace(hz_ctx* h, TP* X, i64 S, i64 zf, i64 zl) {
             if (k > 1 && (p == pfirst[c] || p % k == 0) && (rc = recompute_segment(h, c, p / k, st[c]))) return rc;
             const i64 i = chain_row(h, c, p);
             const double sg = p > pfirst[c] ? -1.0 : 0.0;
-            if ((rc = launch_couple<TP>(h, i, X, S, Y[c], 1, c == 0 ? sg : 0.0, c == 0 ? 0.0 : sg, st[c], 1))) return rc;
-            if ((rc = launch_block_gemm(h, i, (const TP*)Y[c], X, S, 1.0, 0, st[c]))) return rc;
+            if ((rc = launch_couple<TP>(h, i, X, S, Y[c], 1, c == 0 ? sg : 0.0, c == 0 ? 0.0 : sg, st[c], 1, op))) return rc;
+            if ((rc = launch_block_gemm(h, i, (const TP*)Y[c], X, S, 1.0, 0, st[c], op))) return rc;
         }
     }
     HZ_CUDA(h, cudaEventRecord(h->ev_join, st[1]));
     HZ_CUDA(h, cudaStreamWaitEvent(st[0], h->ev_join, 0));
     // middle block
-    if ((rc = launch_couple<TP>(h, mid, X, S, Y[0], 1, top_fwd ? -1.0 : 0.0, bot_fwd ? -1.0 : 0.0, st[0], 1))) return rc;
-    if ((rc = launch_block_gemm(h, mid, (const TP*)Y[0], X, S, 1.0, 0, st[0]))) return rc;
+    if ((rc = launch_couple<TP>(h, mid, X, S, Y[0], 1, top_fwd ? -1.0 : 0.0, bot_fwd ? -1.0 : 0.0, st[0], 1, op))) return rc;
+    if ((rc = launch_block_gemm(h, mid, (const TP*)Y[0], X, S, 1.0, 0, st[0], op))) return rc;
     // back substitution outwards from the middle
     HZ_CUDA(h, cudaEventRecord(h->ev_fork, st[0]));
     HZ_CUDA(h, cudaStreamWaitEvent(st[1], h->ev_fork, 0));
@@ -1602,8 +1612,8 @@ static int solve_inplace(hz_ctx* h, TP* X, i64 S, i64 zf, i64 zl) {
             if (t > len[c]) continue;
             const i64 p = len[c] - t, i = chain_row(h, c, p);
             if (k > 1 && (t == 1 || p % k == k - 1) && (rc = recompute_segment(h, c, p / k, st[c]))) return rc;
-            if ((rc = launch_couple<TP>(h, i, X, S, Y[c], 0, c == 0 ? 0.0 : 1.0, c == 0 ? 1.0 : 0.0, st[c], 0))) return rc;
-            if ((rc = launch_block_gemm(h, i, (const TP*)Y[c], X, S, -1.0, 1, st[c]))) return rc;
+            if ((rc = launch_couple<TP>(h, i, X, S, Y[c], 0, c == 0 ? 0.0 : 1.0, c == 0 ? 1.0 : 0.0, st[c], 0, op))) return rc;
+            if ((rc = launch_block_gemm(h, i, (const TP*)Y[c], X, S, -1.0, 1, st[c], op))) return rc;
         }
     }
     HZ_CUDA(h, cudaEventRecord(h->ev_join, st[1]));
@@ -1618,18 +1628,18 @@ static int solve_inplace(hz_ctx* h, TP* X, i64 S, i64 zf, i64 zl) {
 }
 
 template <class TP>
-static int launch_residual(hz_ctx* h, const TP* X, const TP* Q, i64 S, TP* R) {
+static int launch_residual(hz_ctx* h, const TP* X, const TP* Q, i64 S, TP* R, int op) {
     const int threads = S >= 128 ? 128 : (S >= 64 ? 64 : 32);
     const i64 rows = (i64)h->nf * h->N;
     dim3 grid((unsigned)((S + threads - 1) / threads), (unsigned)(rows < 65535 ? rows : 65535), (unsigned)((rows + 65534) / 65535));
-    auto kfn = residual_kernel<TP>;
+    auto kfn = op == HZ_OP_T ? residual_kernel<TP, 1> : (op == HZ_OP_H ? residual_kernel<TP, 2> : residual_kernel<TP, 0>);
     HZ_LAUNCH_EW(kfn, grid, dim3(threads), 0, h->stream, (const cplx*)h->coef, h->nf, h->nx, h->nz, X, Q, S, R);
     HZ_CHECK_LAUNCH(h);
     return HZ_OK;
 }
 
 template <class TP>
-static int solve_impl(hz_ctx* h, TP* X, int64_t S, double premul_re, double premul_im, int conjugate,
+static int solve_impl(hz_ctx* h, int op, TP* X, int64_t S, double premul_re, double premul_im, int conjugate,
                       int64_t z_first, int64_t z_last, int refine, double* resid_host) {
     const i64 rows = (i64)h->nf * h->N, n = rows * S;
     if (h->ycap < S) {
@@ -1668,12 +1678,12 @@ static int solve_impl(hz_ctx* h, TP* X, int64_t S, double premul_re, double prem
         HZ_LAUNCH_EW(gfn, dim3(blocks_for(rows, 256)), dim3(256), 0, h->stream, (const TP*)X, (i64)S, (i64)0, rows, h->Qprobe);
         HZ_CHECK_LAUNCH(h);
     }
-    int rc = solve_inplace<TP>(h, X, S, z_first, z_last);
+    int rc = solve_inplace<TP>(h, X, S, z_first, z_last, op);
     if (rc) return rc;
     h->probe_pending = false;
     if (probe) {
         HZ_CUDA(h, cudaMemsetAsync(h->d_norm, 0, 2 * sizeof(double), h->stream));
-        auto rfn = residual_col_kernel<TP>;
+        auto rfn = op == HZ_OP_T ? residual_col_kernel<TP, 1> : (op == HZ_OP_H ? residual_col_kernel<TP, 2> : residual_col_kernel<TP, 0>);
         HZ_LAUNCH_IND(rfn, dim3(blocks_for(rows, 256, 148 * 8)), dim3(256), 0, h->stream, (const cplx*)h->coef, h->nf, h->nx, h->nz, (const TP*)X, (i64)S,
                   (i64)0, (const cplx*)h->Qprobe, h->d_norm);
         HZ_CHECK_LAUNCH(h);
@@ -1691,7 +1701,7 @@ static int solve_impl(hz_ctx* h, TP* X, int64_t S, double premul_re, double prem
     }
     double ratio = -1.0;
     for (int it = 0; want_resid; ++it) {
-        if ((rc = launch_residual<TP>(h, X, Qs, S, Rr))) return rc;
+        if ((rc = launch_residual<TP>(h, X, Qs, S, Rr, op))) return rc;
         HZ_CUDA(h, cudaMemsetAsync(h->d_norm, 0, 2 * sizeof(double), h->stream));
         auto nfn = norm2_kernel<TP>;
         HZ_LAUNCH_IND(nfn, dim3(blocks_for(n, 256)), dim3(256), 0, h->stream, (const TP*)Rr, (const TP*)Qs, n, h->d_norm);
@@ -1701,7 +1711,7 @@ static int solve_impl(hz_ctx* h, TP* X, int64_t S, double premul_re, double prem
         HZ_CUDA(h, cudaStreamSynchronize(h->stream));
         ratio = nrm[1] > 0 ? std::sqrt(nrm[0] / nrm[1]) : 0.0;
         if (it >= refine || ratio < 1e-15) break;
-        if ((rc = solve_inplace<TP>(h, Rr, S, -1, -1))) return rc;
+        if ((rc = solve_inplace<TP>(h, Rr, S, -1, -1, op))) return rc;
         auto afn = axpy_kernel<TP>;
         HZ_LAUNCH_EW(afn, dim3(blocks_for(n, 256)), dim3(256), 0, h->stream, X, (const TP*)Rr, n);
         HZ_CHECK_LAUNCH(h);
@@ -1725,20 +1735,28 @@ static int solve_impl(hz_ctx* h, TP* X, int64_t S, double premul_re, double prem
     return HZ_OK;
 }
 
-int hz_solve(hz_handle_t h, void* Xv, int64_t S, double premul_re, double premul_im, int conjugate,
-             int64_t z_first, int64_t z_last, int refine, double* resid_host) {
+int hz_solve_op(hz_handle_t h, int op, void* Xv, int64_t S, double premul_re, double premul_im, int conjugate,
+                int64_t z_first, int64_t z_last, int refine, double* resid_host) {
     if (!h || !Xv) return fail(h, HZ_EINVAL, "hz_solve: NULL argument");
+    if (op != HZ_OP_N && op != HZ_OP_T && op != HZ_OP_H) return fail(h, HZ_EINVAL, "hz_solve_op: op must be HZ_OP_N, HZ_OP_T or HZ_OP_H");
     if (!h->factored) return fail(h, HZ_ESTATE, "hz_solve: call hz_factor first");
     if (S < 1 || S > (1 << 24)) return fail(h, HZ_EINVAL, "hz_solve: S out of range");
     if (refine < -1 || refine > 8) return fail(h, HZ_EINVAL, "hz_solve: refine out of range");
+    if (op != HZ_OP_N && h->dtype == HZ_C64)
+        return fail(h, HZ_ENOTIMPL, "hz_solve_op: transposed solves (HZ_OP_T / HZ_OP_H) are built for complex128 handles only");
     // -1: library default.  The tensor-core (TF32) contraction of the complex64 variant accumulates in the tensor core's
     // truncating FP32 adder (measured ~3.5e-6 per 1000-deep contraction against 3e-7 for FFMA), which over hundreds of
     // block rows exceeds the 1e-4 bound: one refinement step with the FP64 stencil residual restores it.
     if (refine < 0) refine = (h->dtype == HZ_C64 && h->tf32_active) ? 1 : 0;
     HZ_CUDA(h, cudaSetDevice(h->device));
     if (h->dtype == HZ_C64)
-        return solve_impl<cplxf>(h, (cplxf*)Xv, S, premul_re, premul_im, conjugate, z_first, z_last, refine, resid_host);
-    return solve_impl<cplx>(h, (cplx*)Xv, S, premul_re, premul_im, conjugate, z_first, z_last, refine, resid_host);
+        return solve_impl<cplxf>(h, op, (cplxf*)Xv, S, premul_re, premul_im, conjugate, z_first, z_last, refine, resid_host);
+    return solve_impl<cplx>(h, op, (cplx*)Xv, S, premul_re, premul_im, conjugate, z_first, z_last, refine, resid_host);
+}
+
+int hz_solve(hz_handle_t h, void* Xv, int64_t S, double premul_re, double premul_im, int conjugate,
+             int64_t z_first, int64_t z_last, int refine, double* resid_host) {
+    return hz_solve_op(h, HZ_OP_N, Xv, S, premul_re, premul_im, conjugate, z_first, z_last, refine, resid_host);
 }
 
 int hz_profile(hz_handle_t h, int enable, double* out_host) {
@@ -2000,3 +2018,25 @@ int hz_zgemm(int64_t M, int64_t N, int64_t K, double alpha, const void* A, int64
     return HZ_OK;
 }
 
+int hz_zgemm_op(int64_t M, int64_t N, int64_t K, double alpha, const void* A, int64_t lda, int opA, const void* B,
+                int64_t ldb, int beta, void* C, int64_t ldc, int tile, int gemm_3m, void* stream) {
+    if (!A || !B || !C || M < 1 || N < 1 || K < 1) return fail(nullptr, HZ_EINVAL, "hz_zgemm_op: bad argument");
+    if (opA != HZ_OP_N && opA != HZ_OP_T && opA != HZ_OP_H) return fail(nullptr, HZ_EINVAL, "hz_zgemm_op: opA must be HZ_OP_N, HZ_OP_T or HZ_OP_H");
+    if (tile < -1 || tile >= kNumGemmTiles || (gemm_3m != 0 && gemm_3m != 1)) return fail(nullptr, HZ_EINVAL, "hz_zgemm_op: unknown tile or product form");
+    GemmParams p;
+    p.A = (const cplx*)A; p.lda = lda;
+    p.B = (const cplx*)B; p.ldb = ldb;
+    p.C = (cplx*)C; p.ldc = ldc;
+    p.M = (int)M; p.N = (int)N; p.K = (int)K;
+    p.alpha = alpha; p.beta = beta;
+    p.sub_c0 = p.sub_c1 = 0;
+    p.row_nx = 0; p.row_fs = 0;
+    int dev = 0, sms = 148;
+    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int which = zgemm_tile_id(tile >= 0 ? tile : zgemm_pick(p.M, p.N, sms), gemm_3m != 0);
+    if (opA == HZ_OP_T) zgemm_launch<1>(p, (cudaStream_t)stream, sms, which);
+    else if (opA == HZ_OP_H) zgemm_launch<2>(p, (cudaStream_t)stream, sms, which);
+    else zgemm_launch<0>(p, (cudaStream_t)stream, sms, which);
+    HZ_CHECK_LAUNCH(nullptr);
+    return HZ_OK;
+}

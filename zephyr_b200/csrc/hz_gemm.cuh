@@ -12,6 +12,15 @@
 // fragment, and the shared layouts are padded so that every quarter-warp LDS.128 phase is
 // bank-conflict free (A row stride == 4 mod 8 units of 16 B; B row stride == 2 mod 8).
 // Tiles are deliberately small (<= 64x64) so that M x N = 1000 x 512 still fills 144 of 148 SMs.
+//
+// op(A) (template OPA, 0 = N, 1 = T, 2 = C = conjugate transpose): for T and C the stored A is K x M and the kernel
+// computes with op(A)[r][k] = A[k][r] (conjugated for C) -- the transposed / adjoint substitution sweeps apply the
+// stored block inverses S_i^{-1} as S_i^{-T} / S_i^{-H} without a transposed copy.  The A tile is then staged from
+// rows k of the stored A: consecutive threads copy consecutive m of one row (coalesced LDGSTS), into a k-major shared
+// layout sA[k][m] with row stride TM + 2 == 2 (mod 8), the layout of B, so the fragment loads A[g][t] stay conflict
+// free (a quarter-warp phase reads units t*(TM+2) + g, eight distinct banks of 16 B).  C only flips the sign of the
+// imaginary part of the A fragment where it already enters: the -Aim of the four-product form moves to the other
+// term, and the three-product form sums ar - ai instead of ar + ai (epilogue: Re = t1 + t2, Im = s - t1 + t2).
 #pragma once
 #include "hz_platform.h"
 
@@ -44,10 +53,14 @@ struct GemmCfg {
 // M3: three real DMMAs per complex MAC (Re = ar br - ai bi, Im = (ar + ai)(br + bi) - ar br - ai bi) instead of four; the
 // operand sums cost one vector-FP64 add per fragment on a pipe this kernel does not otherwise use.  The kernel is bound
 // by the tensor pipe, so a quarter fewer DMMAs is a quarter less time; normwise accuracy is that of the 4-product form.
-template <int MI, int NI, int WM, int WN, int STAGES, int KS = 1, bool M3 = false>
+template <int MI, int NI, int WM, int WN, int STAGES, int KS = 1, bool M3 = false, int OPA = 0>
 __global__ void __launch_bounds__(32 * WM * WN * KS, 1) zgemm_dmma_kernel(GemmParams p) {
     typedef GemmCfg<MI, NI, WM, WN, STAGES, KS> Cfg;
     constexpr int TM = Cfg::TM, TN = Cfg::TN, NT = Cfg::THREADS, LDB = Cfg::LDB;
+    constexpr bool AT = OPA != 0, ACONJ = OPA == 2;
+    constexpr int LDAT = TM + 2;                                                  // k-major A tile (T, C): == 2 (mod 8)
+    static_assert(OPA >= 0 && OPA <= 2, "op(A) is N, T or C");
+    static_assert(!AT || GEMM_KB * LDAT <= Cfg::A_ELEMS, "the k-major A tile must fit the A stage");
     HZ_SMEM(smem_raw);
     cplx* sA = reinterpret_cast<cplx*>(smem_raw);
     cplx* sB = sA + STAGES * Cfg::A_ELEMS;
@@ -66,18 +79,26 @@ __global__ void __launch_bounds__(32 * WM * WN * KS, 1) zgemm_dmma_kernel(GemmPa
     // copies of the next stage are spread over the k4 steps of the current one, where they fill the issue
     // slot that follows each DMMA, and the addresses are strength-reduced to one base pointer per operand.
     static_assert(NT % GEMM_KB == 0 && NT % TN == 0, "staging assumes whole rows per thread stride");
-    constexpr int NA = (TM * GEMM_KB + NT - 1) / NT, NBL = (GEMM_KB * TN + NT - 1) / NT;
-    constexpr int RA = NT / GEMM_KB, RB = NT / TN;            // row stride between a thread's consecutive copies
-    const int a_r0 = tid / GEMM_KB, a_kk = tid % GEMM_KB;     // A: rows a_r0 + u*RA, fixed column a_kk
+    // A, op N: rows a_r0 + u*RA of the tile, fixed column a_kk.  A, op T/C: k rows a_r0 + u*RA of the stored A, fixed
+    // column a_kk (an m of the tile); RA = NT / TM whole rows per pass, threads past RA * TM rows idle.
+    constexpr int RA = AT ? NT / TM : NT / GEMM_KB, RB = NT / TN;   // row stride between a thread's consecutive copies
+    constexpr int NA = AT ? (GEMM_KB + RA - 1) / RA : (TM * GEMM_KB + NT - 1) / NT, NBL = (GEMM_KB * TN + NT - 1) / NT;
+    const int a_r0 = AT ? tid / TM : tid / GEMM_KB, a_kk = AT ? tid % TM : tid % GEMM_KB;
     const int b_k0 = tid / TN, b_c = tid % TN;                // B: rows b_k0 + u*RB, fixed column b_c
-    const cplx* a_base = p.A + (i64)(m0 + a_r0) * p.lda + a_kk;
+    const cplx* a_base = AT ? p.A + (i64)a_r0 * p.lda + (m0 + a_kk) : p.A + (i64)(m0 + a_r0) * p.lda + a_kk;
     const cplx* b_base = p.B + (i64)b_k0 * p.ldb + (n0 + b_c);
     const i64 a_step = (i64)RA * p.lda, b_step = (i64)RB * p.ldb;
+    const bool a_col_ok = AT && a_r0 < RA && m0 + a_kk < p.M;
     const bool b_col_ok = n0 + b_c < p.N;
     auto stage_op = [&](int op, int k0, cplx* a, cplx* b) {   // op in [0, NA + NBL); everything but k0 folds at compile time
         if (op < NA) {
             const int u = op, r = a_r0 + u * RA;
-            if (u * NT + tid < TM * GEMM_KB) {
+            if constexpr (AT) {
+                if (a_r0 < RA && r < GEMM_KB) {
+                    const bool ok = a_col_ok && (k0 + r < p.K);
+                    cp_async16(a + r * LDAT + a_kk, ok ? a_base + (i64)k0 * p.lda + u * a_step : p.A, ok);
+                }
+            } else if (u * NT + tid < TM * GEMM_KB) {
                 const bool ok = (m0 + r < p.M) && (k0 + a_kk < p.K);
                 cp_async16(a + r * GEMM_LDA + a_kk, ok ? a_base + u * a_step + k0 : p.A, ok);
             }
@@ -119,21 +140,22 @@ __global__ void __launch_bounds__(32 * WM * WN * KS, 1) zgemm_dmma_kernel(GemmPa
         const bool refill = nk < KT;
         cplx* na = sA + (nk % STAGES) * Cfg::A_ELEMS;
         cplx* nb = sB + (nk % STAGES) * Cfg::B_ELEMS;
-        const cplx* a = sA + (kt % STAGES) * Cfg::A_ELEMS + (wm * MI * 8 + g) * GEMM_LDA + t;
+        const cplx* a = AT ? sA + (kt % STAGES) * Cfg::A_ELEMS + t * LDAT + wm * MI * 8 + g
+                           : sA + (kt % STAGES) * Cfg::A_ELEMS + (wm * MI * 8 + g) * GEMM_LDA + t;
         const cplx* b = sB + (kt % STAGES) * Cfg::B_ELEMS + t * LDB + wn * NI * 8 + g;
 #pragma unroll
         for (int k4s = 0; k4s < S4; ++k4s) {
             const int k4 = k4s * KS + wk;
             cplx af[MI], bf[NI];
 #pragma unroll
-            for (int mi = 0; mi < MI; ++mi) af[mi] = a[mi * 8 * GEMM_LDA + k4 * 4];
+            for (int mi = 0; mi < MI; ++mi) af[mi] = AT ? a[k4 * 4 * LDAT + mi * 8] : a[mi * 8 * GEMM_LDA + k4 * 4];
 #pragma unroll
             for (int ni = 0; ni < NI; ++ni) bf[ni] = b[k4 * 4 * LDB + ni * 8];
             // two passes so that consecutive DMMAs never touch the same accumulator
             if constexpr (M3) {
                 double as[MI], bs[NI];
 #pragma unroll
-                for (int mi = 0; mi < MI; ++mi) as[mi] = af[mi].re + af[mi].im;
+                for (int mi = 0; mi < MI; ++mi) as[mi] = ACONJ ? af[mi].re - af[mi].im : af[mi].re + af[mi].im;
 #pragma unroll
                 for (int ni = 0; ni < NI; ++ni) bs[ni] = bf[ni].re + bf[ni].im;
 #pragma unroll
@@ -167,8 +189,8 @@ __global__ void __launch_bounds__(32 * WM * WN * KS, 1) zgemm_dmma_kernel(GemmPa
             for (int mi = 0; mi < MI; ++mi)
 #pragma unroll
                 for (int ni = 0; ni < NI; ++ni) {
-                    dmma884(cre[mi][ni][0], cre[mi][ni][1], -af[mi].im, bf[ni].im);
-                    dmma884(cim[mi][ni][0], cim[mi][ni][1], af[mi].im, bf[ni].re);
+                    dmma884(cre[mi][ni][0], cre[mi][ni][1], ACONJ ? af[mi].im : -af[mi].im, bf[ni].im);
+                    dmma884(cim[mi][ni][0], cim[mi][ni][1], ACONJ ? -af[mi].im : af[mi].im, bf[ni].re);
                 }
             }
         }
@@ -183,8 +205,8 @@ __global__ void __launch_bounds__(32 * WM * WN * KS, 1) zgemm_dmma_kernel(GemmPa
 #pragma unroll
                 for (int j = 0; j < 2; ++j) {
                     const double t1 = cre[mi][ni][j], t2 = c2[mi][ni][j];
-                    cre[mi][ni][j] = t1 - t2;
-                    cim[mi][ni][j] = cim[mi][ni][j] - t1 - t2;
+                    cre[mi][ni][j] = ACONJ ? t1 + t2 : t1 - t2;
+                    cim[mi][ni][j] = ACONJ ? cim[mi][ni][j] - t1 + t2 : cim[mi][ni][j] - t1 - t2;
                 }
     }
     if (KS > 1) {
@@ -243,10 +265,10 @@ __global__ void __launch_bounds__(32 * WM * WN * KS, 1) zgemm_dmma_kernel(GemmPa
 }
 
 // ---- host-side dispatch -------------------------------------------------------------------
-template <int MI, int NI, int WM, int WN, int STAGES, int KS = 1, bool M3 = false>
+template <int MI, int NI, int WM, int WN, int STAGES, int KS = 1, bool M3 = false, int OPA = 0>
 static inline int zgemm_launch_cfg(const GemmParams& p, cudaStream_t stream) {
     typedef GemmCfg<MI, NI, WM, WN, STAGES, KS> Cfg;
-    auto kfn = zgemm_dmma_kernel<MI, NI, WM, WN, STAGES, KS, M3>;
+    auto kfn = zgemm_dmma_kernel<MI, NI, WM, WN, STAGES, KS, M3, OPA>;
     static std::atomic<unsigned long long> configured{0};
     hz_once_per_device(configured, [&]() { cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM); });
     dim3 grid((p.N + Cfg::TN - 1) / Cfg::TN, (p.M + Cfg::TM - 1) / Cfg::TM, 1);
@@ -273,48 +295,68 @@ static inline int zgemm_pick(int M, int N, int num_sms) {
     return besti;
 }
 
-// every instance zgemm_launch can pick, for the eager kernel preload (hz_api.cu: preload_all_kernels)
-template <class F>
-static inline void zgemm_for_each_instance(F f) {
-    f(zgemm_dmma_kernel<4, 2, 2, 4, 3>); f(zgemm_dmma_kernel<7, 1, 1, 8, 3>); f(zgemm_dmma_kernel<6, 1, 1, 8, 3>); f(zgemm_dmma_kernel<5, 1, 1, 8, 3>);
-    f(zgemm_dmma_kernel<2, 2, 2, 4, 4>); f(zgemm_dmma_kernel<2, 1, 2, 4, 4>); f(zgemm_dmma_kernel<1, 1, 2, 4, 4>); f(zgemm_dmma_kernel<7, 1, 1, 8, 3, 2>);
-    f(zgemm_dmma_kernel<4, 2, 2, 4, 3, 2>); f(zgemm_dmma_kernel<6, 1, 1, 8, 3, 2>); f(zgemm_dmma_kernel<5, 1, 1, 8, 3, 2>); f(zgemm_dmma_kernel<7, 2, 1, 4, 3>);
-    f(zgemm_dmma_kernel<7, 2, 1, 4, 3, 2>);
-    // three-multiplication twins of the tiles zgemm_pick chooses from
-    f(zgemm_dmma_kernel<4, 2, 2, 4, 3, 1, true>); f(zgemm_dmma_kernel<7, 1, 1, 8, 3, 1, true>); f(zgemm_dmma_kernel<6, 1, 1, 8, 3, 1, true>);
-    f(zgemm_dmma_kernel<5, 1, 1, 8, 3, 1, true>); f(zgemm_dmma_kernel<2, 2, 2, 4, 4, 1, true>); f(zgemm_dmma_kernel<2, 1, 2, 4, 4, 1, true>);
-    f(zgemm_dmma_kernel<1, 1, 2, 4, 4, 1, true>);
-    f(zgemm_dmma_kernel<7, 2, 1, 4, 3, 1, true>); f(zgemm_dmma_kernel<7, 2, 1, 4, 3, 2, true>); f(zgemm_dmma_kernel<7, 1, 1, 8, 3, 2, true>);
+// kernel instance (tile id of zgemm_launch) for candidate tiling `cand` of kGemmTiles and the product form; m3 ids are
+// 16 + cand, except 56 x 64: warps of 56 x 16 need fewer operand sums per DMMA (109 vs 111 us at 1000 x 512 x 1000)
+static inline int zgemm_tile_id(int cand, bool m3) {
+    const int which = cand + (m3 ? 16 : 0);
+    return which == 17 ? 24 : which;
 }
 
-// m3: three-multiplication complex products (tiles 16 + i are the M3 twins of the auto-picked tiles 0..6)
-static inline int zgemm_launch(const GemmParams& p, cudaStream_t stream, int num_sms, int force_tile = -1, bool m3 = false) {
-    int which = force_tile >= 0 ? force_tile : zgemm_pick(p.M, p.N, num_sms) + (m3 ? 16 : 0);
-    if (force_tile < 0 && which == 17) which = 24;      // 56 x 64: warps of 56 x 16 need fewer operand sums per DMMA (109 vs 111 us at 1000 x 512 x 1000)
-    switch (which) {
-        case 16: return zgemm_launch_cfg<4, 2, 2, 4, 3, 1, true>(p, stream);
-        case 17: return zgemm_launch_cfg<7, 1, 1, 8, 3, 1, true>(p, stream);
-        case 18: return zgemm_launch_cfg<6, 1, 1, 8, 3, 1, true>(p, stream);
-        case 19: return zgemm_launch_cfg<5, 1, 1, 8, 3, 1, true>(p, stream);
-        case 20: return zgemm_launch_cfg<2, 2, 2, 4, 4, 1, true>(p, stream);
-        case 21: return zgemm_launch_cfg<2, 1, 2, 4, 4, 1, true>(p, stream);
-        case 22: return zgemm_launch_cfg<1, 1, 2, 4, 4, 1, true>(p, stream);
-        case 23: return zgemm_launch_cfg<7, 2, 1, 4, 3, 1, true>(p, stream);   // M3 twins of 11, 12 and 7 (fewer operand sums per DMMA / split-K)
-        case 24: return zgemm_launch_cfg<7, 2, 1, 4, 3, 2, true>(p, stream);
-        case 25: return zgemm_launch_cfg<7, 1, 1, 8, 3, 2, true>(p, stream);
-        case 0: return zgemm_launch_cfg<4, 2, 2, 4, 3>(p, stream);   // 64 x 64
-        case 1: return zgemm_launch_cfg<7, 1, 1, 8, 3>(p, stream);   // 56 x 64
-        case 2: return zgemm_launch_cfg<6, 1, 1, 8, 3>(p, stream);   // 48 x 64
-        case 3: return zgemm_launch_cfg<5, 1, 1, 8, 3>(p, stream);   // 40 x 64
-        case 4: return zgemm_launch_cfg<2, 2, 2, 4, 4>(p, stream);   // 32 x 64
-        case 5: return zgemm_launch_cfg<2, 1, 2, 4, 4>(p, stream);   // 32 x 32
-        case 6: return zgemm_launch_cfg<1, 1, 2, 4, 4>(p, stream);   // 16 x 32
-        case 7: return zgemm_launch_cfg<7, 1, 1, 8, 3, 2>(p, stream);   // 56 x 64, 16 warps (split-K)
-        case 8: return zgemm_launch_cfg<4, 2, 2, 4, 3, 2>(p, stream);   // 64 x 64, 16 warps (split-K)
-        case 9: return zgemm_launch_cfg<6, 1, 1, 8, 3, 2>(p, stream);   // 48 x 64, 16 warps
-        case 10: return zgemm_launch_cfg<5, 1, 1, 8, 3, 2>(p, stream);  // 40 x 64, 16 warps
-        case 11: return zgemm_launch_cfg<7, 2, 1, 4, 3>(p, stream);     // 56 x 64, 4 warps of 56 x 16
-        case 12: return zgemm_launch_cfg<7, 2, 1, 4, 3, 2>(p, stream);  // 56 x 64, 8 warps of 56 x 16 (split-K)
-        default: return zgemm_launch_cfg<1, 1, 2, 4, 4>(p, stream);
+// every instance zgemm_launch can pick for op(A) = OPA (for OPA = 0 also the study tiles), for the eager kernel preload
+// (hz_api.cu: preload_all_kernels)
+template <int OPA, class F>
+static inline void zgemm_for_each_instance(F f) {
+    f(zgemm_dmma_kernel<4, 2, 2, 4, 3, 1, false, OPA>); f(zgemm_dmma_kernel<7, 1, 1, 8, 3, 1, false, OPA>);
+    f(zgemm_dmma_kernel<6, 1, 1, 8, 3, 1, false, OPA>); f(zgemm_dmma_kernel<5, 1, 1, 8, 3, 1, false, OPA>);
+    f(zgemm_dmma_kernel<2, 2, 2, 4, 4, 1, false, OPA>); f(zgemm_dmma_kernel<2, 1, 2, 4, 4, 1, false, OPA>);
+    f(zgemm_dmma_kernel<1, 1, 2, 4, 4, 1, false, OPA>);
+    // three-multiplication twins of the tiles zgemm_pick chooses from
+    f(zgemm_dmma_kernel<4, 2, 2, 4, 3, 1, true, OPA>); f(zgemm_dmma_kernel<6, 1, 1, 8, 3, 1, true, OPA>);
+    f(zgemm_dmma_kernel<5, 1, 1, 8, 3, 1, true, OPA>); f(zgemm_dmma_kernel<2, 2, 2, 4, 4, 1, true, OPA>);
+    f(zgemm_dmma_kernel<2, 1, 2, 4, 4, 1, true, OPA>); f(zgemm_dmma_kernel<1, 1, 2, 4, 4, 1, true, OPA>);
+    f(zgemm_dmma_kernel<7, 2, 1, 4, 3, 2, true, OPA>);
+    if constexpr (OPA == 0) {
+        f(zgemm_dmma_kernel<7, 1, 1, 8, 3, 2>); f(zgemm_dmma_kernel<4, 2, 2, 4, 3, 2>); f(zgemm_dmma_kernel<6, 1, 1, 8, 3, 2>);
+        f(zgemm_dmma_kernel<5, 1, 1, 8, 3, 2>); f(zgemm_dmma_kernel<7, 2, 1, 4, 3>); f(zgemm_dmma_kernel<7, 2, 1, 4, 3, 2>);
+        f(zgemm_dmma_kernel<7, 1, 1, 8, 3, 1, true>); f(zgemm_dmma_kernel<7, 2, 1, 4, 3, 1, true>); f(zgemm_dmma_kernel<7, 1, 1, 8, 3, 2, true>);
     }
+}
+
+// m3: three-multiplication complex products (tiles 16 + i are the M3 twins of the auto-picked tiles 0..6).  op(A) T and C
+// (OPA 1, 2) exist for the tiles the host picks (zgemm_tile_id); the study tiles 7..12, 17, 23, 25 are op N only.
+template <int OPA = 0>
+static inline int zgemm_launch(const GemmParams& p, cudaStream_t stream, int num_sms, int force_tile = -1, bool m3 = false) {
+    const int which = force_tile >= 0 ? force_tile : zgemm_tile_id(zgemm_pick(p.M, p.N, num_sms), m3);
+    switch (which) {
+        case 16: return zgemm_launch_cfg<4, 2, 2, 4, 3, 1, true, OPA>(p, stream);
+        case 18: return zgemm_launch_cfg<6, 1, 1, 8, 3, 1, true, OPA>(p, stream);
+        case 19: return zgemm_launch_cfg<5, 1, 1, 8, 3, 1, true, OPA>(p, stream);
+        case 20: return zgemm_launch_cfg<2, 2, 2, 4, 4, 1, true, OPA>(p, stream);
+        case 21: return zgemm_launch_cfg<2, 1, 2, 4, 4, 1, true, OPA>(p, stream);
+        case 22: return zgemm_launch_cfg<1, 1, 2, 4, 4, 1, true, OPA>(p, stream);
+        case 24: return zgemm_launch_cfg<7, 2, 1, 4, 3, 2, true, OPA>(p, stream);   // M3 twin of 12 (56 x 64, warps of 56 x 16, split-K)
+        case 0: return zgemm_launch_cfg<4, 2, 2, 4, 3, 1, false, OPA>(p, stream);   // 64 x 64
+        case 1: return zgemm_launch_cfg<7, 1, 1, 8, 3, 1, false, OPA>(p, stream);   // 56 x 64
+        case 2: return zgemm_launch_cfg<6, 1, 1, 8, 3, 1, false, OPA>(p, stream);   // 48 x 64
+        case 3: return zgemm_launch_cfg<5, 1, 1, 8, 3, 1, false, OPA>(p, stream);   // 40 x 64
+        case 4: return zgemm_launch_cfg<2, 2, 2, 4, 4, 1, false, OPA>(p, stream);   // 32 x 64
+        case 5: return zgemm_launch_cfg<2, 1, 2, 4, 4, 1, false, OPA>(p, stream);   // 32 x 32
+        case 6: return zgemm_launch_cfg<1, 1, 2, 4, 4, 1, false, OPA>(p, stream);   // 16 x 32
+        default: break;
+    }
+    if constexpr (OPA == 0) {
+        switch (which) {
+            case 17: return zgemm_launch_cfg<7, 1, 1, 8, 3, 1, true>(p, stream);
+            case 23: return zgemm_launch_cfg<7, 2, 1, 4, 3, 1, true>(p, stream);   // M3 twins of 11 and 7 (fewer operand sums per DMMA / split-K)
+            case 25: return zgemm_launch_cfg<7, 1, 1, 8, 3, 2, true>(p, stream);
+            case 7: return zgemm_launch_cfg<7, 1, 1, 8, 3, 2>(p, stream);   // 56 x 64, 16 warps (split-K)
+            case 8: return zgemm_launch_cfg<4, 2, 2, 4, 3, 2>(p, stream);   // 64 x 64, 16 warps (split-K)
+            case 9: return zgemm_launch_cfg<6, 1, 1, 8, 3, 2>(p, stream);   // 48 x 64, 16 warps
+            case 10: return zgemm_launch_cfg<5, 1, 1, 8, 3, 2>(p, stream);  // 40 x 64, 16 warps
+            case 11: return zgemm_launch_cfg<7, 2, 1, 4, 3>(p, stream);     // 56 x 64, 4 warps of 56 x 16
+            case 12: return zgemm_launch_cfg<7, 2, 1, 4, 3, 2>(p, stream);  // 56 x 64, 8 warps of 56 x 16 (split-K)
+            default: break;
+        }
+    }
+    return zgemm_launch_cfg<1, 1, 2, 4, 4, 1, false, OPA>(p, stream);
 }

@@ -11,9 +11,20 @@
 #include "hz_factor.cuh"
 #include "hz_c64.cuh"
 
-// Y[rl][s] = use_self * X_i[rl][s] + sgn_lo * (A_{i,i-1} X_{i-1})[rl][s] + sgn_hi * (A_{i,i+1} X_{i+1})[rl][s]
+// Entry of op(A) (OP: 0 = N, 1 = T, 2 = H) in row (fr, node), column (fc, nbr = node + dz*nx + dx), slot = (dz+1)*3 + dx+1.
+// The transposed stencil is a gather: A^T[r][c] = A[c][r] is stored at the neighbour node, in the mirrored slot (8 - slot)
+// of the swapped field pair (fc, fr); H conjugates it.  Block-wise this makes (A^T)_{i,i-1} = U_{i-1}^T and
+// (A^T)_{i,i+1} = L_{i+1}^T, so the sweeps below keep their structure for every op.
+template <int OP>
+__device__ __forceinline__ cplx op_coef(const cplx* __restrict__ coef, int nf, int fr, int fc, int slot, i64 node, i64 nbr, i64 N) {
+    if constexpr (OP == 0) return coef_plane(coef, nf, fr, fc, slot, N)[node];
+    const cplx v = coef_plane(coef, nf, fc, fr, 8 - slot, N)[nbr];
+    return OP == 2 ? cconj(v) : v;
+}
+
+// Y[rl][s] = use_self * X_i[rl][s] + sgn_lo * (op(A)_{i,i-1} X_{i-1})[rl][s] + sgn_hi * (op(A)_{i,i+1} X_{i+1})[rl][s]
 // rl = f*nx + ix indexes the block-local row; Y is a dense b x S buffer (ld = S).
-template <class TP>
+template <class TP, int OP = 0>
 __global__ void couple_kernel(const cplx* __restrict__ coef, int nf, int nx, int nz, int i,
                               const TP* __restrict__ X, i64 S, TP* __restrict__ Y,
                               int use_self, double sgn_lo, double sgn_hi) {
@@ -34,8 +45,9 @@ __global__ void couple_kernel(const cplx* __restrict__ coef, int nf, int nx, int
 #pragma unroll
             for (int a = -1; a <= 1; ++a) {
                 if (ix + a < 0 || ix + a >= nx) continue;
-                const cplx cf = coef_plane(coef, nf, fr, fc, (dzs + 1) * 3 + a + 1, N)[node];
-                cfma(part, cf, ldp(&X[((i64)fc * N + (i64)(i + dzs) * nx + ix + a) * S + s]));
+                const i64 nbr = (i64)(i + dzs) * nx + ix + a;
+                const cplx cf = op_coef<OP>(coef, nf, fr, fc, (dzs + 1) * 3 + a + 1, node, nbr, N);
+                cfma(part, cf, ldp(&X[((i64)fc * N + nbr) * S + s]));
             }
         }
         acc = acc + sg * part;
@@ -43,8 +55,8 @@ __global__ void couple_kernel(const cplx* __restrict__ coef, int nf, int nx, int
     stp(&Y[(i64)rl * S + s], acc);
 }
 
-// R = Q - A X over the whole panel (stencil SpMM); one thread per (row, s)
-template <class TP>
+// R = Q - op(A) X over the whole panel (stencil SpMM); one thread per (row, s)
+template <class TP, int OP = 0>
 __global__ void residual_kernel(const cplx* __restrict__ coef, int nf, int nx, int nz,
                                 const TP* __restrict__ X, const TP* __restrict__ Q, i64 S,
                                 TP* __restrict__ R) {
@@ -64,8 +76,9 @@ __global__ void residual_kernel(const cplx* __restrict__ coef, int nf, int nx, i
 #pragma unroll
             for (int a = -1; a <= 1; ++a) {
                 if (ix + a < 0 || ix + a >= nx) continue;
-                const cplx cf = coef_plane(coef, nf, fr, fc, (dzs + 1) * 3 + a + 1, N)[node];
-                const cplx xv = ldp(&X[((i64)fc * N + node + (i64)dzs * nx + a) * S + s]);
+                const i64 nbr = node + (i64)dzs * nx + a;
+                const cplx cf = op_coef<OP>(coef, nf, fr, fc, (dzs + 1) * 3 + a + 1, node, nbr, N);
+                const cplx xv = ldp(&X[((i64)fc * N + nbr) * S + s]);
                 acc = acc - cf * xv;
             }
         }
@@ -77,8 +90,8 @@ template <class TP>
 __global__ void gather_col_kernel(const TP* __restrict__ X, i64 S, i64 col, i64 rows, cplx* __restrict__ out) {
     for (i64 r = (i64)blockIdx.x * blockDim.x + threadIdx.x; r < rows; r += (i64)gridDim.x * blockDim.x) out[r] = ldp(&X[r * S + col]);
 }
-// ... and afterwards out[0] += ||q - A x||^2, out[1] += ||q||^2 for that column (9-point stencil residual in FP64)
-template <class TP>
+// ... and afterwards out[0] += ||q - op(A) x||^2, out[1] += ||q||^2 for that column (9-point stencil residual in FP64)
+template <class TP, int OP = 0>
 __global__ void residual_col_kernel(const cplx* __restrict__ coef, int nf, int nx, int nz, const TP* __restrict__ X, i64 S, i64 col,
                                     const cplx* __restrict__ q, double* __restrict__ out) {
     const i64 N = (i64)nx * nz, rows = (i64)nf * N;
@@ -96,8 +109,9 @@ __global__ void residual_col_kernel(const cplx* __restrict__ coef, int nf, int n
 #pragma unroll
                 for (int a = -1; a <= 1; ++a) {
                     if (ix + a < 0 || ix + a >= nx) continue;
-                    const cplx cf = coef_plane(coef, nf, fr, fc, (dzs + 1) * 3 + a + 1, N)[node];
-                    acc = acc - cf * ldp(&X[((i64)fc * N + node + (i64)dzs * nx + a) * S + col]);
+                    const i64 nbr = node + (i64)dzs * nx + a;
+                    const cplx cf = op_coef<OP>(coef, nf, fr, fc, (dzs + 1) * 3 + a + 1, node, nbr, N);
+                    acc = acc - cf * ldp(&X[((i64)fc * N + nbr) * S + col]);
                 }
             }
         sr += cabs2(acc);

@@ -158,6 +158,10 @@ class BaseDiscretization(BaseModelDependent):
     def refine(self):
         return int(getattr(self, '_refine', -1))            # -1: library default (hz_solve)
 
+    def _refine_steps(self, op):
+        """Refinement steps of a solve with op(A) (HZ_OP_N / T / H)."""
+        return self.refine
+
     @property
     def shape(self):
         n = self._nf * self.nrow
@@ -392,24 +396,32 @@ class BaseDiscretization(BaseModelDependent):
             zr = (-1, -1)
         return X, zr
 
-    def solve_device(self, X, zrange=(-1, -1), conjugate=True, want_residual=False):
-        """In place on a device panel X (nf*N, S): X <- conj(premul * A^-1 X).  Fast path for
+    def solve_device(self, X, zrange=(-1, -1), conjugate=True, want_residual=False, trans='N'):
+        """In place on a device panel X (nf*N, S): X <- conj(premul * op(A)^-1 X) with op(A) = A, A^T or A^H for
+        ``trans`` = 'N', 'T' or 'H' (all three from the same factors; 'T' / 'H' need complex128).  Fast path for
         callers that keep wavefields in HBM (survey / bench)."""
         lib = _lib.get_lib()
+        op = _lib.trans_op(trans)
         if X.dtype != self.panel_dtype or not X.is_contiguous():
             raise ValueError('panel must be a contiguous %s tensor' % (self.panel_dtype,))
         self._ensure_factors(*zrange)
         self._bind_stream()
         pm = complex(self.premul)
         res = C.c_double(-1.0)
-        _lib.check(lib.hz_solve(self.handle, _lib.ptr(X), X.shape[1], pm.real, pm.imag, int(bool(conjugate)),
-                                int(zrange[0]), int(zrange[1]), self.refine,
-                                C.byref(res) if (want_residual or self.refine > 0) else None), self.handle)
-        if want_residual or self.refine > 0:
+        refine = self._refine_steps(op)
+        _lib.check(lib.hz_solve_op(self.handle, op, _lib.ptr(X), X.shape[1], pm.real, pm.imag, int(bool(conjugate)),
+                                   int(zrange[0]), int(zrange[1]), refine,
+                                   C.byref(res) if (want_residual or refine > 0) else None), self.handle)
+        if want_residual or refine > 0:
             self.last_residual = res.value
         return X
 
-    def __mul__(self, rhs):
+    def solve(self, rhs, trans='N'):
+        """conj(premul * op(A)^-1 rhs) for an ndarray / scipy.sparse right-hand side, op(A) = A, A^T, A^H for
+        ``trans`` = 'N', 'T', 'H' (scipy's ``SuperLU.solve`` convention), with the conventions of ``Disc * rhs``
+        (premul, conjugation, Eurus' zero padding of N-row right-hand sides and clipping of the result).
+        ``solve(rhs)`` is ``Disc * rhs``."""
+        _lib.trans_op(trans)
         squeeze = False
         if not sp.issparse(rhs):
             rhs = np.asarray(rhs)
@@ -418,10 +430,13 @@ class BaseDiscretization(BaseModelDependent):
                 squeeze = True
         clip = self._rows_ok(rhs.shape[0])
         X, zr = self.rhs_to_device(rhs)
-        self.solve_device(X, zr)
+        self.solve_device(X, zr, trans=trans)
         out = X[:self.nrow] if clip else X
         res = _panel_to_host(out)
         return res[:, 0] if squeeze else res
+
+    def __mul__(self, rhs):
+        return self.solve(rhs)
 
     def __call__(self, value):
         return self * value
@@ -458,7 +473,8 @@ class MiniZephyr25D(BaseDiscretization):
     """2.5-D modelling: Fourier summation of 2-D solves over cross-line wavenumbers ky
     (zephyr/backend/minizephyr.py:346-460).  Each ky is its own operator (own factorisation); the
     partial wavefields are accumulated on the device and only the sum is copied back.  ``parallel``
-    is accepted and ignored; factors are released after each ky unless ``keepFactors`` is set."""
+    is accepted and ignored; factors are released after each ky unless ``keepFactors`` is set.  Transposed solves
+    (``solve(rhs, trans='T' / 'H')``) are not built for the 2.5-D sum; ``solve(rhs)`` is ``self * rhs``."""
 
     initMap = {
         'Disc':         (False,     '_Disc',        None),
@@ -477,6 +493,11 @@ class MiniZephyr25D(BaseDiscretization):
 
     def _default_mord(self):
         return (self.nx, +1)
+
+    def solve(self, rhs, trans='N'):
+        if _lib.trans_op(trans) != _lib.HZ_OP_N:
+            raise NotImplementedError('MiniZephyr25D: transposed solves are not built for the 2.5-D sum')
+        return self * rhs
 
     @property
     def Disc(self):
@@ -574,6 +595,14 @@ class Eurus(BaseDiscretization, BaseAnisotropic):
     @property
     def refine(self):
         return int(getattr(self, '_refine', 1))
+
+    def _refine_steps(self, op):
+        """Transposed solves (A^T, A^H) refine twice by default: on ill-conditioned TTI operators the transposed sweep
+        leaves about five times the N sweep's residual after one step (measured at 200 x 400: 5e-11 - 1.2e-10 against
+        1.3e-11 - 1.7e-11), two steps bring it to ~1.5e-12.  A `refine` set in systemConfig is used as given."""
+        if op != _lib.HZ_OP_N and not hasattr(self, '_refine'):
+            return 2
+        return self.refine
 
     def _create_args(self):
         return float(self.cPML)

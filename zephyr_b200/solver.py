@@ -6,7 +6,8 @@ with the assembled sparse matrix and must return an object with ``solve(rhs)``. 
 the 9-diagonal matrices MiniZephyr builds (and Eurus' 2N x 2N block form) and solves with the GPU block
 factorisation -- for A/B runs of the factorisation alone: assembly stays in the reference (SURVEY.md 8(b) explains
 why the full path plugs in at 'Disc' instead).  No conjugation and no premul here: that is the caller's job
-(discretization.py:103), exactly as with splu.
+(discretization.py:103), exactly as with splu.  ``solve(rhs, trans)`` takes SuperLU's ``trans`` ('N', 'T', 'H': solve
+with A, A^T or A^H) and runs all three from the same factors (complex128 only for 'T' / 'H').
 """
 import ctypes as C
 
@@ -57,9 +58,10 @@ class BlockTridiagonalSolver(object):
         _lib.check(lib.hz_set_coefficients(h, _lib.ptr(np.ascontiguousarray(planes))), h)
         _lib.check(lib.hz_factor(h, -1), h)
 
-    def solve(self, rhs):
+    def solve(self, rhs, trans='N'):
         import torch
         lib = _lib.get_lib()
+        op = _lib.trans_op(trans)
         rhs = np.asarray(rhs.toarray() if sp.issparse(rhs) else rhs, dtype=np.complex128)
         squeeze = rhs.ndim < 2
         if squeeze:
@@ -68,7 +70,7 @@ class BlockTridiagonalSolver(object):
             raise ValueError('dimension mismatch')
         X = torch.from_numpy(np.ascontiguousarray(rhs)).to(self._dev, copy=True).to(torch.complex64 if self._c64 else torch.complex128)
         _lib.check(lib.hz_set_stream(self._handle, _lib.current_stream_ptr(self._dev)), self._handle)
-        _lib.check(lib.hz_solve(self._handle, _lib.ptr(X), X.shape[1], 1.0, 0.0, 0, -1, -1, -1, None), self._handle)
+        _lib.check(lib.hz_solve_op(self._handle, op, _lib.ptr(X), X.shape[1], 1.0, 0.0, 0, -1, -1, -1, None), self._handle)
         out = X.to(torch.complex128).cpu().numpy()
         return out[:, 0] if squeeze else out
 
