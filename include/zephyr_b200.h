@@ -199,6 +199,17 @@ int hz_gradient(const void* uF, const void* uB, int64_t N, int64_t S, const void
 /* a11: phi += 0.5*||wd (d - dobs)||^2 ; v = wd*wd*(d - dobs) (v may be NULL).                    */
 int hz_misfit(const void* d, const void* dobs, int64_t n, double wd, void* v, double* phi, void* stream);
 
+/* Adjoint-state gradient of MiniZephyr (DESIGN.md §2).  hz_stencil_xcorr: the stencil cross-correlation of an adjoint
+ * panel lam and a forward panel u (both complex128, N x S, N = nx*nz, row-major), u as the forward solve returns it
+ * (conjugated):  G[slot*N + i] = sum_s lam[i*S + s] * conj(u[(i + off(slot))*S + s]),  off(slot) = (slot/3 - 1)*nx +
+ * (slot%3 - 1); G is 9*N complex128, overwritten, zero on boundary rows.
+ * hz_assemble_vjp: the vector-Jacobian product of the handle's last hz_assemble with G, added into g_c and g_rho
+ * (float64, N; either may be NULL, not both):  g_c[n] -= Re(alpha[n] sum_{slot,i} G[slot][i] d coef[slot][i] / d c[n]),
+ * g_rho[n] -= Re(sum G d coef / d rho[n]).  alpha (complex128, N) may be NULL (1).  On the handle's stream.  Complex64
+ * and Eurus handles: HZ_ENOTIMPL; coefficients loaded with hz_set_coefficients: HZ_ESTATE.                        */
+int hz_stencil_xcorr(const void* lam, const void* u, int64_t nx, int64_t nz, int64_t S, void* G, void* stream);
+int hz_assemble_vjp(hz_handle_t h, const void* G, const void* alpha, double* g_c, double* g_rho);
+
 /* complex64 variant (hz_create(dtype = HZ_C64)): block inverses are stored in complex64 (planar: a real and an
  * imaginary float32 plane per block) and applied by the tcgen05 tensor cores: kind::tf32 MMAs with 3xTF32 operand
  * splitting (FP32-like products), tiles staged by TMA, accumulators in TMEM, split-K partial sums combined with

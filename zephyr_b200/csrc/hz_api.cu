@@ -19,6 +19,7 @@
 #include "hz_tf32.cuh"
 #include "hz_solve.cuh"
 #include "hz_survey.cuh"
+#include "hz_adjoint.cuh"
 #include "../../include/zephyr_b200.h"
 
 // sampled device timing of the contraction kernel (every PROF_EVERY-th launch is bracketed by
@@ -43,6 +44,8 @@ struct hz_ctx {
     double* binv = nullptr;      // per-node buoyancy 1/rho
     cplx* pmltab = nullptr;      // Eurus: 3*nx + 3*nz PML reciprocal tables
     bool have_model = false, assembled = false, factored = false;
+    AsmParams asm_p;             // parameters of the last hz_assemble (the adjoint-gradient VJP recomputes from them)
+    bool asm_from_model = false; // false after hz_set_coefficients: the planes are no longer a function of the model
     // factors and workspaces
     cplx* Sinv = nullptr;        // complex128 block inverses (HZ_C128)
     cplxf* Sinv64 = nullptr;     // complex64 block inverses (HZ_C64)
@@ -411,6 +414,8 @@ int hz_assemble(hz_handle_t h, double freq_re, double freq_im, double tau, doubl
     HZ_CHECK_LAUNCH(h);
     h->assembled = true;
     h->factored = false;
+    h->asm_p = p;
+    h->asm_from_model = true;
     return HZ_OK;
 }
 
@@ -423,6 +428,7 @@ int hz_set_coefficients(hz_handle_t h, const void* planes_host) {
     HZ_CUDA(h, cudaStreamSynchronize(h->stream));
     h->assembled = true;
     h->factored = false;
+    h->asm_from_model = false;
     return HZ_OK;
 }
 
@@ -1090,6 +1096,7 @@ static void preload_factor_kernels() {
     preload_kernel(gj_post_quit2_kernel);
     preload_kernel(node_terms_kernel); preload_kernel(assemble_mz_kernel); preload_kernel(eurus_pml_tables_kernel); preload_kernel(assemble_eurus_kernel);
     preload_kernel(nearest_index_kernel); preload_kernel(kaiser_taps_kernel);
+    preload_kernel(stencil_xcorr_kernel); preload_kernel(assemble_mz_vjp_kernel);
     preload_panel_kernels<cplx>();
     preload_panel_kernels<cplxf>();
     zgemm_for_each_instance<0>([](auto kfn) { preload_kernel(kfn); });
@@ -1969,6 +1976,32 @@ int hz_misfit(const void* d, const void* dobs, int64_t n, double wd, void* v, do
 }
 int hz_misfit_c64(const void* d, const void* dobs, int64_t n, double wd, void* v, double* phi, void* stream) {
     return misfit_impl<cplxf>(d, dobs, n, wd, v, phi, stream);
+}
+
+int hz_stencil_xcorr(const void* lam, const void* u, int64_t nx, int64_t nz, int64_t S, void* G, void* stream) {
+    if (!lam || !u || !G) return fail(nullptr, HZ_EINVAL, "hz_stencil_xcorr: NULL argument");
+    if (nx < 3 || nz < 3 || nx > 32768 || nz > (1 << 24) || S < 1) return fail(nullptr, HZ_EINVAL, "hz_stencil_xcorr: nx, nz or S out of range");
+    const int threads = 256;
+    const i64 wpb = threads / 32, N = nx * nz;
+    HZ_LAUNCH_IND(stencil_xcorr_kernel, dim3(blocks_for((N + wpb - 1) / wpb * threads, threads, 148 * 16)), dim3(threads), 0, (cudaStream_t)stream,
+                  (const cplx*)lam, (const cplx*)u, (int)nx, (int)nz, (i64)S, (cplx*)G);
+    HZ_CHECK_LAUNCH(nullptr);
+    return HZ_OK;
+}
+
+int hz_assemble_vjp(hz_handle_t h, const void* G, const void* alpha, double* g_c, double* g_rho) {
+    if (!h) return fail(h, HZ_EINVAL, "hz_assemble_vjp: NULL handle");
+    if (h->disc != HZ_DISC_MINIZEPHYR || h->dtype != HZ_C128)
+        return fail(h, HZ_ENOTIMPL, "hz_assemble_vjp: built for complex128 MiniZephyr handles only");
+    if (!G || (!g_c && !g_rho)) return fail(h, HZ_EINVAL, "hz_assemble_vjp: G and at least one of g_c, g_rho are required");
+    if (!h->assembled || !h->asm_from_model)
+        return fail(h, HZ_ESTATE, "hz_assemble_vjp: the coefficients must come from hz_assemble of the current model");
+    HZ_CUDA(h, cudaSetDevice(h->device));
+    const int threads = 128;
+    HZ_LAUNCH_EW(assemble_mz_vjp_kernel, dim3((unsigned)((h->N + threads - 1) / threads)), dim3(threads), 0, h->stream, (const cplx*)h->c,
+                 (const cplx*)h->Kp, (const double*)h->binv, (const cplx*)G, (const cplx*)alpha, h->asm_p, g_c, g_rho);
+    HZ_CHECK_LAUNCH(h);
+    return HZ_OK;
 }
 
 int hz_cgemm_tf32(int64_t M, int64_t N, int64_t K, double alpha, const float* A_planes, int64_t lda, const float* Y_planes, int64_t ldy,

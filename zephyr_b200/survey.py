@@ -14,6 +14,7 @@ import scipy.sparse as sp
 
 from . import _lib, parallel
 from .base import AttributeMapper, BaseModelDependent
+from .discretization import MiniZephyr
 from .distributors import MultiFreq, ViscoMultiFreq
 from .source import SparseKaiserSource
 
@@ -415,8 +416,9 @@ class HelmBaseProblem(BaseModelDependent):
                                               _lib.current_stream_ptr(ops['dev'])))
         return d
 
-    def backproject_device(self, ifreq, v, out=None):
-        """uB = Disc * (rVec.T v) for one frequency; v is the (R, S) device residual."""
+    def backproject_device(self, ifreq, v, out=None, vals=None, conjugate=True, trans='N'):
+        """uB = Disc * (rVec.T v) for one frequency; v is the (R, S) device residual.  `vals` replaces the receiver
+        taps (the CSR values of the back-projection operator); `conjugate` and `trans` are passed to solve_device."""
         import torch
         ops = self._device_ops()
         sub = self.system.subProblems[ifreq]
@@ -424,14 +426,16 @@ class HelmBaseProblem(BaseModelDependent):
         X = out if out is not None else torch.empty((sub.shape[1], sv.nsrc), dtype=sub.panel_dtype, device=ops['dev'])
         X.zero_()
         if ops['mode'] != 'fixed':
-            _lib.check(_lib.panel_fn('hz_spmm_percol', sub.c64)(1, sv.nrec * sv.nsrc, _lib.ptr(ops['r_ptr']), _lib.ptr(ops['r_col']), _lib.ptr(ops['r_val']),
+            _lib.check(_lib.panel_fn('hz_spmm_percol', sub.c64)(1, sv.nrec * sv.nsrc, _lib.ptr(ops['r_ptr']), _lib.ptr(ops['r_col']),
+                                                             _lib.ptr(ops['r_val'] if vals is None else vals),
                                                              sv.nsrc, _lib.ptr(v), _lib.ptr(X), sv.nsrc, _lib.current_stream_ptr(ops['dev'])))
-            sub.solve_device(X, ops['b_z'])
+            sub.solve_device(X, ops['b_z'], conjugate=conjugate, trans=trans)
             return X
-        _lib.check(_lib.panel_fn('hz_spmm_csr', sub.c64)(ops['b_nodes'].numel(), _lib.ptr(ops['b_ptr']), _lib.ptr(ops['b_col']), _lib.ptr(ops['b_val']),
+        _lib.check(_lib.panel_fn('hz_spmm_csr', sub.c64)(ops['b_nodes'].numel(), _lib.ptr(ops['b_ptr']), _lib.ptr(ops['b_col']),
+                                              _lib.ptr(ops['b_val'] if vals is None else vals),
                                               _lib.ptr(ops['b_nodes']), _lib.ptr(v), sv.nsrc, sv.nsrc, _lib.ptr(X), sv.nsrc, 1, 0,
                                               _lib.current_stream_ptr(ops['dev'])))
-        sub.solve_device(X, ops['b_z'])
+        sub.solve_device(X, ops['b_z'], conjugate=conjugate, trans=trans)
         return X
 
     def _panel_bytes(self):
@@ -561,6 +565,117 @@ class HelmBaseProblem(BaseModelDependent):
         host = red.cpu().numpy()
         return float(host[N]), host[:N].copy()
 
+    # ---- adjoint-state gradient (DESIGN.md §2) ------------------------------------------------
+    def _adjoint_alpha(self, ifreq):
+        """dc_f/dc at every node for frequency ifreq as a host complex array, or None when c_f = c."""
+        return None
+
+    def _check_adjoint_supported(self):
+        subs = self.system.subProblems
+        for i in self.system.localFreqIndices:
+            sub = subs[i]
+            if not isinstance(sub, MiniZephyr):
+                raise NotImplementedError('misfit_and_adjoint_gradient is built for the MiniZephyr operator only, not %s'
+                                          % type(sub).__name__)
+            if sub.c64:
+                raise NotImplementedError("misfit_and_adjoint_gradient needs complex128 factors (A^T solves); dtype='complex64' "
+                                          'has no transposed solve')
+
+    def _adjoint_taps(self, ifreq):
+        """Receiver taps of the adjoint source of one frequency: conjugated (rterms may be complex) and divided by
+        premul, so that the premultiplied, unconjugated A^T solve of the back-projection returns lambda = A^-T (Rv^H v)
+        itself.  Formed on the caller's stream, before any worker stream reads them."""
+        ops = self._device_ops()
+        key = 'b_val' if ops['mode'] == 'fixed' else 'r_val'
+        if key + '_conj' not in ops:
+            ops[key + '_conj'] = ops[key].conj().resolve_conj()
+        pm = complex(self.system.subProblems[ifreq].premul)
+        return ops[key + '_conj'] if pm == 1 else ops[key + '_conj'] / pm
+
+    def misfit_and_adjoint_gradient(self, dobs, Wd=1., wrt=('c',), to_host=True):
+        """phi = 0.5 ||Wd (dpred - dobs)||^2 and its exact gradient with respect to the model parameters named in
+        ``wrt`` ('c', 'rho'), by the adjoint-state method: per frequency a forward solve, an A^T solve of the
+        back-projected residual, the stencil cross-correlation of the two panels and the vector-Jacobian product of
+        the assembly (DESIGN.md §2).  Unlike ``misfit_and_gradient``, which follows the reference's Jtvec formula,
+        this is the derivative of phi: what a line search or a quasi-Newton method needs.
+
+        Returns (phi, {'c': g_c, 'rho': g_rho}) with the requested keys only (float64 arrays of N).  For the viscous
+        problem g_c is with respect to the real base velocity; where rho is not given (Gardner's rule rho = 310
+        Re(c)^0.25), g_c includes the change of rho with c and g_rho is the partial derivative at fixed c.  dobs: the
+        (R, S, F) data or the device tensor from ``upload_dobs``.  to_host=False returns the all-reduced device
+        tensor [g_wrt[0] (N), g_wrt[1] (N), ..., phi] (float64) instead.  MiniZephyr operators in complex128 only."""
+        import torch
+        wrt = tuple(wrt)
+        if not wrt or len(set(wrt)) != len(wrt) or any(k not in ('c', 'rho') for k in wrt):
+            raise ValueError("wrt must name 'c' and/or 'rho', each at most once")
+        self._check_adjoint_supported()
+        ops = self._device_ops()
+        dev, sv, N = ops['dev'], self.survey, self.nrow
+        nx, nz = int(self.nx), int(self.nz)
+        local = self.system.localFreqIndices
+        subs = self.system.subProblems
+        do_all = dobs if isinstance(dobs, torch.Tensor) else self.upload_dobs(dobs)
+        workers = self._workers(ops['s_z'])
+        gardner = self.systemConfig.get('rho', None) is None
+        want_c, want_rho = 'c' in wrt, 'rho' in wrt
+        rho_scratch = want_rho or (gardner and want_c)
+        lib = _lib.get_lib()
+
+        def to_dev(a, dt):
+            return torch.from_numpy(np.ascontiguousarray(a, dtype=dt).ravel()).to(dev)
+        # everything the workers share or only read is formed here, on the caller's stream, which every worker stream
+        # waits for when it starts (MultiFreq.run_local)
+        taps = {i: self._adjoint_taps(i) for i in local}
+        alphas = {i: (None if self._adjoint_alpha(i) is None else to_dev(self._adjoint_alpha(i), np.complex128)) for i in local}
+        drho_dc = {}
+        if gardner and want_c:
+            # rho_f = 310 Re(c_f)^0.25 and Re(c_f) = Re(alpha_f) c  =>  drho_f/dc = rho_f / (4 Re(c))
+            cr = np.real(np.asarray(self.systemConfig['c'], dtype=np.complex128)) * np.ones((nz, nx))
+            drho_dc = {i: to_dev(0.25 * np.asarray(subs[i].rho, dtype=np.float64).reshape((nz, nx)) / cr, np.float64) for i in local}
+        accs, phis, panels = {}, {}, {}
+
+        def one(ifreq, slot):
+            stream = _lib.current_stream_ptr(dev)
+            if slot not in accs:
+                accs[slot] = {k: torch.zeros((N,), dtype=torch.float64, device=dev) for k in wrt}
+                phis[slot] = torch.zeros((1,), dtype=torch.float64, device=dev)
+                panels[slot] = {'uF': None, 'lam': None, 'G': torch.empty((9 * N,), dtype=torch.complex128, device=dev),
+                                'grho': torch.empty((N,), dtype=torch.float64, device=dev) if rho_scratch else None}
+            pn = panels[slot]
+            sub = subs[ifreq]
+            self._ensure_factors(ifreq, ops['s_z'], evict=workers == 1)
+            uF = pn['uF'] = self.forward_device(ifreq, out=pn['uF'])
+            d = self.extract_device(uF)
+            do = do_all[local.index(ifreq)]
+            v = torch.empty_like(d)
+            _lib.check(lib.hz_misfit(_lib.ptr(d), _lib.ptr(do), d.numel(), float(Wd), _lib.ptr(v), _lib.ptr(phis[slot]), stream))
+            lam = pn['lam'] = self.backproject_device(ifreq, v, out=pn['lam'], vals=taps[ifreq], conjugate=False, trans='T')
+            _lib.check(lib.hz_stencil_xcorr(_lib.ptr(lam), _lib.ptr(uF), nx, nz, sv.nsrc, _lib.ptr(pn['G']), stream))
+            sub._bind_stream()
+            g_c = accs[slot]['c'] if want_c else None
+            if rho_scratch:
+                pn['grho'].zero_()
+            _lib.check(lib.hz_assemble_vjp(sub.handle, _lib.ptr(pn['G']), _lib.ptr(alphas[ifreq]), _lib.ptr(g_c), _lib.ptr(pn['grho'])), sub.handle)
+            if want_rho:
+                accs[slot]['rho'] += pn['grho']
+            if drho_dc:
+                accs[slot]['c'] += pn['grho'] * drho_dc[ifreq]
+            if not self.system.keepFactors:
+                del sub.factors
+            return None
+        self.system.run_local(one, workers=workers, bytes_per_worker=2 * self._panel_bytes() + 160 * N if local else 0)
+        nk = len(wrt)
+        red = torch.zeros((nk * N + 1,), dtype=torch.float64, device=dev)
+        for slot in accs:
+            for j, k in enumerate(wrt):
+                red[j * N:(j + 1) * N] += accs[slot][k]
+            red[nk * N] += phis[slot][0]
+        parallel.allreduce_sum_(red)
+        if not to_host:
+            return red
+        host = red.cpu().numpy()
+        return float(host[nk * N]), {k: host[j * N:(j + 1) * N].copy() for j, k in enumerate(wrt)}
+
 
 class Helm2DProblem(HelmBaseProblem):
     SystemWrapper = MultiFreq
@@ -568,3 +683,12 @@ class Helm2DProblem(HelmBaseProblem):
 
 class Helm2DViscoProblem(HelmBaseProblem):
     SystemWrapper = ViscoMultiFreq
+
+    def _adjoint_alpha(self, ifreq):
+        """c_f = fact_f c (1 + i/(2Q)) (ViscoMultiFreq.spUpdates), so dc_f/dc = fact_f (1 + i/(2Q))."""
+        system = self.system
+        Q = np.asarray(system.Q, dtype=np.float64).reshape((int(self.nz), int(self.nx)))
+        alpha = 1. + 0.5j / Q
+        if system.disperseFreqs:
+            alpha = alpha * (1. + (np.log(system.freqs[ifreq] / system.freqBase) / (np.pi * Q)))
+        return alpha
