@@ -210,6 +210,21 @@ int hz_misfit(const void* d, const void* dobs, int64_t n, double wd, void* v, do
 int hz_stencil_xcorr(const void* lam, const void* u, int64_t nx, int64_t nz, int64_t S, void* G, void* stream);
 int hz_assemble_vjp(hz_handle_t h, const void* G, const void* alpha, double* g_c, double* g_rho);
 
+/* Born modelling of MiniZephyr (DESIGN.md §2, "Born modelling and Gauss-Newton products"); the exact transposes of the
+ * two entries above.  hz_assemble_jvp: the Jacobian-vector product of the handle's last hz_assemble along a real model
+ * perturbation dc, drho (float64, N; either may be NULL, not both):  dcoef[slot*N + i] = sum_n (d coef[slot][i] / d c[n])
+ * alpha[n] dc[n] + (d coef[slot][i] / d rho[n]) drho[n], 9*N complex128 in the layout of the assembled planes,
+ * overwritten, zero on boundary rows.  alpha (complex128, N) may be NULL (1).  For any G,
+ * Re sum G dcoef = -(g_c . dc + g_rho . drho) with g_c, g_rho from hz_assemble_vjp.  On the handle's stream; the same
+ * refusals as hz_assemble_vjp.
+ * hz_stencil_apply: the tangent stencil applied to a forward panel u (complex128, N x S, as the forward solve returns it):
+ * out[i*S + s] = scale * sum_slot dcoef[slot*N + i] * conj(u[(i + off(slot))*S + s]), zero on boundary rows; out must
+ * not overlap u.  With scale = -1/premul, the conjugating solve (hz_solve, conjugate = 1) of out returns the Born field
+ * conj(-A^-1 dA w).  Duality with hz_stencil_xcorr: sum lam .* out = scale sum G .* dcoef.                         */
+int hz_assemble_jvp(hz_handle_t h, const double* dc, const double* drho, const void* alpha, void* dcoef);
+int hz_stencil_apply(const void* dcoef, const void* u, int64_t nx, int64_t nz, int64_t S, double scale_re, double scale_im,
+                     void* out, void* stream);
+
 /* complex64 variant (hz_create(dtype = HZ_C64)): block inverses are stored in complex64 (planar: a real and an
  * imaginary float32 plane per block) and applied by the tcgen05 tensor cores: kind::tf32 MMAs with 3xTF32 operand
  * splitting (FP32-like products), tiles staged by TMA, accumulators in TMEM, split-K partial sums combined with

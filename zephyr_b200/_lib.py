@@ -56,6 +56,8 @@ SIGNATURES = {
     'hz_misfit': (_int, [_vp, _vp, _i64, _f64, _vp, _vp, _vp]),
     'hz_stencil_xcorr': (_int, [_vp, _vp, _i64, _i64, _i64, _vp, _vp]),
     'hz_assemble_vjp': (_int, [_vp, _vp, _vp, _vp, _vp]),
+    'hz_stencil_apply': (_int, [_vp, _vp, _i64, _i64, _i64, _f64, _f64, _vp, _vp]),
+    'hz_assemble_jvp': (_int, [_vp, _vp, _vp, _vp, _vp]),
     'hz_scatter_coo_c64': (_int, [_vp, _i64, _i64, _vp, _vp, _vp, _f64, _f64, _vp]),
     'hz_spmm_csr_c64': (_int, [_i64, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp, _i64, _i64, _int, _vp]),
     'hz_gradient_c64': (_int, [_vp, _vp, _i64, _i64, _vp, _vp, _vp]),

@@ -20,6 +20,7 @@
 #include "hz_solve.cuh"
 #include "hz_survey.cuh"
 #include "hz_adjoint.cuh"
+#include "hz_born.cuh"
 #include "../../include/zephyr_b200.h"
 
 // sampled device timing of the contraction kernel (every PROF_EVERY-th launch is bracketed by
@@ -1097,6 +1098,7 @@ static void preload_factor_kernels() {
     preload_kernel(node_terms_kernel); preload_kernel(assemble_mz_kernel); preload_kernel(eurus_pml_tables_kernel); preload_kernel(assemble_eurus_kernel);
     preload_kernel(nearest_index_kernel); preload_kernel(kaiser_taps_kernel);
     preload_kernel(stencil_xcorr_kernel); preload_kernel(assemble_mz_vjp_kernel);
+    preload_kernel(stencil_apply_kernel); preload_kernel(assemble_mz_jvp_kernel);
     preload_panel_kernels<cplx>();
     preload_panel_kernels<cplxf>();
     zgemm_for_each_instance<0>([](auto kfn) { preload_kernel(kfn); });
@@ -2000,6 +2002,33 @@ int hz_assemble_vjp(hz_handle_t h, const void* G, const void* alpha, double* g_c
     const int threads = 128;
     HZ_LAUNCH_EW(assemble_mz_vjp_kernel, dim3((unsigned)((h->N + threads - 1) / threads)), dim3(threads), 0, h->stream, (const cplx*)h->c,
                  (const cplx*)h->Kp, (const double*)h->binv, (const cplx*)G, (const cplx*)alpha, h->asm_p, g_c, g_rho);
+    HZ_CHECK_LAUNCH(h);
+    return HZ_OK;
+}
+
+int hz_stencil_apply(const void* dcoef, const void* u, int64_t nx, int64_t nz, int64_t S, double scale_re, double scale_im, void* out,
+                     void* stream) {
+    if (!dcoef || !u || !out) return fail(nullptr, HZ_EINVAL, "hz_stencil_apply: NULL argument");
+    if (nx < 3 || nz < 3 || nx > 32768 || nz > (1 << 24) || S < 1) return fail(nullptr, HZ_EINVAL, "hz_stencil_apply: nx, nz or S out of range");
+    const int tx = S >= 256 ? 256 : (int)((S + 31) / 32 * 32), ty = 256 / tx;
+    const i64 N = nx * nz;
+    HZ_LAUNCH_IND(stencil_apply_kernel, dim3(blocks_for(N, STENCIL_APPLY_RUN * ty, (i64)1 << 24)), dim3(tx, ty), 0, (cudaStream_t)stream,
+                  (const cplx*)dcoef, (const cplx*)u, (int)nx, (int)nz, (i64)S, mk(scale_re, scale_im), (cplx*)out);
+    HZ_CHECK_LAUNCH(nullptr);
+    return HZ_OK;
+}
+
+int hz_assemble_jvp(hz_handle_t h, const double* dc, const double* drho, const void* alpha, void* dcoef) {
+    if (!h) return fail(h, HZ_EINVAL, "hz_assemble_jvp: NULL handle");
+    if (h->disc != HZ_DISC_MINIZEPHYR || h->dtype != HZ_C128)
+        return fail(h, HZ_ENOTIMPL, "hz_assemble_jvp: built for complex128 MiniZephyr handles only");
+    if (!dcoef || (!dc && !drho)) return fail(h, HZ_EINVAL, "hz_assemble_jvp: dcoef and at least one of dc, drho are required");
+    if (!h->assembled || !h->asm_from_model)
+        return fail(h, HZ_ESTATE, "hz_assemble_jvp: the coefficients must come from hz_assemble of the current model");
+    HZ_CUDA(h, cudaSetDevice(h->device));
+    const int threads = 128;
+    HZ_LAUNCH_EW(assemble_mz_jvp_kernel, dim3((unsigned)((h->N + threads - 1) / threads)), dim3(threads), 0, h->stream, (const cplx*)h->c,
+                 (const cplx*)h->Kp, (const double*)h->binv, dc, drho, (const cplx*)alpha, h->asm_p, (cplx*)dcoef);
     HZ_CHECK_LAUNCH(h);
     return HZ_OK;
 }

@@ -153,25 +153,28 @@ class HelmBaseSurvey(AttributeMapper):
             if hasattr(self.prob, 'dpred_device'):
                 # same result as projecting lazyFields(m); the wavefields stay in HBM and only the
                 # (nrec, nsrc, nfreq) data cube crosses PCIe (summed over frequency shards)
-                import torch
                 self.prob.updateModel(m)
-                dd = self.prob.dpred_device()
-                dev = self.prob._device_ops()['dev']
-                rank, world = parallel.rank_world()
-                # every rank contributes only the (R, S) slabs of its own frequencies: all-gather of
-                # ceil(F / world) slabs per rank instead of all-reducing a cube that is zero elsewhere
-                per = -(-self.nfreq // world)
-                mine = torch.zeros((per, self.nrec, self.nsrc), dtype=torch.complex128, device=dev)
-                for k, ifreq in enumerate(sorted(dd)):
-                    mine[k] = dd[ifreq].to(torch.complex128)
-                slabs = parallel.allgather(mine)                  # list over ranks of (per, R, S)
-                cube = torch.empty((self.nrec, self.nsrc, self.nfreq), dtype=torch.complex128, device=dev)
-                for r, slab in enumerate(slabs):
-                    for k, ifreq in enumerate(parallel.shard_indices(self.nfreq, r, world)):
-                        cube[:, :, ifreq] = slab[k]
-                return cube.cpu().numpy().ravel()
+                return self._gather_freqs(self.prob.dpred_device()).cpu().numpy().ravel()
             u = self.prob.lazyFields(m)
         return self.projectFields(u).ravel()
+
+    def _gather_freqs(self, dd):
+        """{ifreq: (R, S) device tensor} of this rank's frequencies -> the (R, S, F) complex128 device cube on every rank.
+        Every rank contributes only the (R, S) slabs of its own frequencies: all-gather of ceil(F / world) slabs per
+        rank instead of all-reducing a cube that is zero elsewhere."""
+        import torch
+        dev = self.prob._device_ops()['dev']
+        rank, world = parallel.rank_world()
+        per = -(-self.nfreq // world)
+        mine = torch.zeros((per, self.nrec, self.nsrc), dtype=torch.complex128, device=dev)
+        for k, ifreq in enumerate(sorted(dd)):
+            mine[k] = dd[ifreq].to(torch.complex128)
+        slabs = parallel.allgather(mine)                  # list over ranks of (per, R, S)
+        cube = torch.empty((self.nrec, self.nsrc, self.nfreq), dtype=torch.complex128, device=dev)
+        for r, slab in enumerate(slabs):
+            for k, ifreq in enumerate(parallel.shard_indices(self.nfreq, r, world)):
+                cube[:, :, ifreq] = slab[k]
+        return cube
 
     @property
     def postProcessors(self):
@@ -570,16 +573,15 @@ class HelmBaseProblem(BaseModelDependent):
         """dc_f/dc at every node for frequency ifreq as a host complex array, or None when c_f = c."""
         return None
 
-    def _check_adjoint_supported(self):
+    def _check_adjoint_supported(self, name='misfit_and_adjoint_gradient'):
         subs = self.system.subProblems
         for i in self.system.localFreqIndices:
             sub = subs[i]
             if not isinstance(sub, MiniZephyr):
-                raise NotImplementedError('misfit_and_adjoint_gradient is built for the MiniZephyr operator only, not %s'
-                                          % type(sub).__name__)
+                raise NotImplementedError('%s is built for the MiniZephyr operator only, not %s' % (name, type(sub).__name__))
             if sub.c64:
-                raise NotImplementedError("misfit_and_adjoint_gradient needs complex128 factors (A^T solves); dtype='complex64' "
-                                          'has no transposed solve')
+                raise NotImplementedError("%s needs complex128 factors (A^T solves); dtype='complex64' has no transposed solve"
+                                          % name)
 
     def _adjoint_taps(self, ifreq):
         """Receiver taps of the adjoint source of one frequency: conjugated (rterms may be complex) and divided by
@@ -591,6 +593,123 @@ class HelmBaseProblem(BaseModelDependent):
             ops[key + '_conj'] = ops[key].conj().resolve_conj()
         pm = complex(self.system.subProblems[ifreq].premul)
         return ops[key + '_conj'] if pm == 1 else ops[key + '_conj'] / pm
+
+    @staticmethod
+    def _check_wrt(wrt):
+        wrt = tuple(wrt)
+        if not wrt or len(set(wrt)) != len(wrt) or any(k not in ('c', 'rho') for k in wrt):
+            raise ValueError("wrt must name 'c' and/or 'rho', each at most once")
+        return wrt
+
+    def _check_dm(self, dm, wrt):
+        """A model perturbation {name: N float64 values} over exactly the names of ``wrt`` -> host float64 arrays of N."""
+        if not isinstance(dm, dict) or set(dm) != set(wrt):
+            raise ValueError('dm must be a dict with exactly the keys %s' % (wrt,))
+        out = {}
+        for k in wrt:
+            a = np.asarray(dm[k])
+            if np.iscomplexobj(a) or a.size != self.nrow:
+                raise ValueError("dm['%s'] must hold %d real values" % (k, self.nrow))
+            out[k] = np.ascontiguousarray(a, dtype=np.float64).ravel()
+        return out
+
+    def _derivative_sweep(self, wrt, adjoint_data, dm=None, back=True, nextra=0):
+        """The per-frequency device pipeline of the exact derivatives (DESIGN.md §2).  For every local frequency:
+
+        1. the forward panel uF (``forward_device``);
+        2. if ``dm`` is given, the Born panel dU = conj(-A^-1 dA w) in a second panel: ``hz_assemble_jvp`` along dm,
+           ``hz_stencil_apply`` with scale -1/premul and an N solve over the whole depth range;
+        3. v = adjoint_data(ifreq, uF, dU, extra), an (R, S) device tensor (extra: this worker's float64 accumulator
+           of ``nextra`` values);
+        4. if ``back``: lambda = A^-T (Rv^H v) (back-projection with the adjoint taps, A^T solve), ``hz_stencil_xcorr``
+           of lambda and uF and ``hz_assemble_vjp`` into per-worker accumulators of -Re sum lambda^T (dA/dm) w.
+
+        The caller checks that the operators are supported.  ``dm`` holds float64 device tensors of N over ``wrt``.  Where rho is not given (Gardner's rule), the tangent
+        and the gradient both carry density's dependence on c.  Returns {ifreq: v} if not ``back``; otherwise the
+        float64 device tensor [g_wrt[0] (N), g_wrt[1] (N), ..., extra] summed over the workers of this rank (the
+        caller all-reduces it)."""
+        import torch
+        ops = self._device_ops()
+        dev, sv, N = ops['dev'], self.survey, self.nrow
+        nx, nz = int(self.nx), int(self.nz)
+        local = self.system.localFreqIndices
+        subs = self.system.subProblems
+        workers = self._workers(ops['s_z'])
+        gardner = self.systemConfig.get('rho', None) is None
+        want_c, want_rho = 'c' in wrt, 'rho' in wrt
+        rho_scratch = back and (want_rho or (gardner and want_c))
+        tan_rho = dm is not None and gardner and want_c          # the tangent's drho_f = drho_f/dc dc (+ drho)
+        lib = _lib.get_lib()
+
+        def to_dev(a, dt):
+            return torch.from_numpy(np.ascontiguousarray(a, dtype=dt).ravel()).to(dev)
+        # everything the workers share or only read is formed here, on the caller's stream, which every worker stream
+        # waits for when it starts (MultiFreq.run_local)
+        taps = {i: self._adjoint_taps(i) for i in local} if back else {}
+        alphas = {i: (None if self._adjoint_alpha(i) is None else to_dev(self._adjoint_alpha(i), np.complex128)) for i in local}
+        drho_dc = {}
+        if gardner and want_c:
+            # rho_f = 310 Re(c_f)^0.25 and Re(c_f) = Re(alpha_f) c  =>  drho_f/dc = rho_f / (4 Re(c))
+            cr = np.real(np.asarray(self.systemConfig['c'], dtype=np.complex128)) * np.ones((nz, nx))
+            drho_dc = {i: to_dev(0.25 * np.asarray(subs[i].rho, dtype=np.float64).reshape((nz, nx)) / cr, np.float64) for i in local}
+        accs, extras, panels = {}, {}, {}
+
+        def one(ifreq, slot):
+            stream = _lib.current_stream_ptr(dev)
+            if slot not in panels:
+                if back:
+                    accs[slot] = {k: torch.zeros((N,), dtype=torch.float64, device=dev) for k in wrt}
+                extras[slot] = torch.zeros((nextra,), dtype=torch.float64, device=dev)
+                panels[slot] = {'uF': None, 'lam': None, 'G': torch.empty((9 * N,), dtype=torch.complex128, device=dev),
+                                'grho': torch.empty((N,), dtype=torch.float64, device=dev) if rho_scratch else None,
+                                'drho': torch.empty((N,), dtype=torch.float64, device=dev) if tan_rho else None}
+            pn = panels[slot]
+            sub = subs[ifreq]
+            self._ensure_factors(ifreq, ops['s_z'], evict=workers == 1)
+            uF = pn['uF'] = self.forward_device(ifreq, out=pn['uF'])
+            dU = None
+            if dm is not None:
+                dc, drho = dm.get('c'), dm.get('rho')
+                if tan_rho:
+                    drho = torch.mul(drho_dc[ifreq], dc, out=pn['drho']) if drho is None else \
+                        torch.addcmul(drho, drho_dc[ifreq], dc, out=pn['drho'])
+                sub._bind_stream()
+                _lib.check(lib.hz_assemble_jvp(sub.handle, _lib.ptr(dc), _lib.ptr(drho), _lib.ptr(alphas[ifreq]), _lib.ptr(pn['G'])),
+                           sub.handle)
+                if pn['lam'] is None:
+                    pn['lam'] = torch.empty_like(uF)
+                scale = -1. / complex(sub.premul)
+                _lib.check(lib.hz_stencil_apply(_lib.ptr(pn['G']), _lib.ptr(uF), nx, nz, sv.nsrc, scale.real, scale.imag,
+                                                _lib.ptr(pn['lam']), stream))
+                dU = sub.solve_device(pn['lam'], (-1, -1))          # the secondary source fills every depth
+            v = adjoint_data(ifreq, uF, dU, extras[slot])
+            if back:
+                lam = pn['lam'] = self.backproject_device(ifreq, v, out=pn['lam'], vals=taps[ifreq], conjugate=False, trans='T')
+                _lib.check(lib.hz_stencil_xcorr(_lib.ptr(lam), _lib.ptr(uF), nx, nz, sv.nsrc, _lib.ptr(pn['G']), stream))
+                sub._bind_stream()
+                g_c = accs[slot]['c'] if want_c else None
+                if rho_scratch:
+                    pn['grho'].zero_()
+                _lib.check(lib.hz_assemble_vjp(sub.handle, _lib.ptr(pn['G']), _lib.ptr(alphas[ifreq]), _lib.ptr(g_c), _lib.ptr(pn['grho'])),
+                           sub.handle)
+                if want_rho:
+                    accs[slot]['rho'] += pn['grho']
+                if drho_dc:
+                    accs[slot]['c'] += pn['grho'] * drho_dc[ifreq]
+            if not self.system.keepFactors:
+                del sub.factors
+            return None if back else v
+        per_worker = 2 * self._panel_bytes() + 160 * N + (8 * N if tan_rho else 0)
+        res = self.system.run_local(one, workers=workers, bytes_per_worker=per_worker if local else 0)
+        if not back:
+            return res
+        nk = len(wrt)
+        red = torch.zeros((nk * N + nextra,), dtype=torch.float64, device=dev)
+        for slot in accs:
+            for j, k in enumerate(wrt):
+                red[j * N:(j + 1) * N] += accs[slot][k]
+            red[nk * N:] += extras[slot]
+        return red
 
     def misfit_and_adjoint_gradient(self, dobs, Wd=1., wrt=('c',), to_host=True):
         """phi = 0.5 ||Wd (dpred - dobs)||^2 and its exact gradient with respect to the model parameters named in
@@ -605,77 +724,81 @@ class HelmBaseProblem(BaseModelDependent):
         (R, S, F) data or the device tensor from ``upload_dobs``.  to_host=False returns the all-reduced device
         tensor [g_wrt[0] (N), g_wrt[1] (N), ..., phi] (float64) instead.  MiniZephyr operators in complex128 only."""
         import torch
-        wrt = tuple(wrt)
-        if not wrt or len(set(wrt)) != len(wrt) or any(k not in ('c', 'rho') for k in wrt):
-            raise ValueError("wrt must name 'c' and/or 'rho', each at most once")
+        wrt = self._check_wrt(wrt)
         self._check_adjoint_supported()
-        ops = self._device_ops()
-        dev, sv, N = ops['dev'], self.survey, self.nrow
-        nx, nz = int(self.nx), int(self.nz)
         local = self.system.localFreqIndices
-        subs = self.system.subProblems
         do_all = dobs if isinstance(dobs, torch.Tensor) else self.upload_dobs(dobs)
-        workers = self._workers(ops['s_z'])
-        gardner = self.systemConfig.get('rho', None) is None
-        want_c, want_rho = 'c' in wrt, 'rho' in wrt
-        rho_scratch = want_rho or (gardner and want_c)
         lib = _lib.get_lib()
+        dev = self._device_ops()['dev']
 
-        def to_dev(a, dt):
-            return torch.from_numpy(np.ascontiguousarray(a, dtype=dt).ravel()).to(dev)
-        # everything the workers share or only read is formed here, on the caller's stream, which every worker stream
-        # waits for when it starts (MultiFreq.run_local)
-        taps = {i: self._adjoint_taps(i) for i in local}
-        alphas = {i: (None if self._adjoint_alpha(i) is None else to_dev(self._adjoint_alpha(i), np.complex128)) for i in local}
-        drho_dc = {}
-        if gardner and want_c:
-            # rho_f = 310 Re(c_f)^0.25 and Re(c_f) = Re(alpha_f) c  =>  drho_f/dc = rho_f / (4 Re(c))
-            cr = np.real(np.asarray(self.systemConfig['c'], dtype=np.complex128)) * np.ones((nz, nx))
-            drho_dc = {i: to_dev(0.25 * np.asarray(subs[i].rho, dtype=np.float64).reshape((nz, nx)) / cr, np.float64) for i in local}
-        accs, phis, panels = {}, {}, {}
-
-        def one(ifreq, slot):
-            stream = _lib.current_stream_ptr(dev)
-            if slot not in accs:
-                accs[slot] = {k: torch.zeros((N,), dtype=torch.float64, device=dev) for k in wrt}
-                phis[slot] = torch.zeros((1,), dtype=torch.float64, device=dev)
-                panels[slot] = {'uF': None, 'lam': None, 'G': torch.empty((9 * N,), dtype=torch.complex128, device=dev),
-                                'grho': torch.empty((N,), dtype=torch.float64, device=dev) if rho_scratch else None}
-            pn = panels[slot]
-            sub = subs[ifreq]
-            self._ensure_factors(ifreq, ops['s_z'], evict=workers == 1)
-            uF = pn['uF'] = self.forward_device(ifreq, out=pn['uF'])
+        def residual(ifreq, uF, dU, phi):
             d = self.extract_device(uF)
             do = do_all[local.index(ifreq)]
             v = torch.empty_like(d)
-            _lib.check(lib.hz_misfit(_lib.ptr(d), _lib.ptr(do), d.numel(), float(Wd), _lib.ptr(v), _lib.ptr(phis[slot]), stream))
-            lam = pn['lam'] = self.backproject_device(ifreq, v, out=pn['lam'], vals=taps[ifreq], conjugate=False, trans='T')
-            _lib.check(lib.hz_stencil_xcorr(_lib.ptr(lam), _lib.ptr(uF), nx, nz, sv.nsrc, _lib.ptr(pn['G']), stream))
-            sub._bind_stream()
-            g_c = accs[slot]['c'] if want_c else None
-            if rho_scratch:
-                pn['grho'].zero_()
-            _lib.check(lib.hz_assemble_vjp(sub.handle, _lib.ptr(pn['G']), _lib.ptr(alphas[ifreq]), _lib.ptr(g_c), _lib.ptr(pn['grho'])), sub.handle)
-            if want_rho:
-                accs[slot]['rho'] += pn['grho']
-            if drho_dc:
-                accs[slot]['c'] += pn['grho'] * drho_dc[ifreq]
-            if not self.system.keepFactors:
-                del sub.factors
-            return None
-        self.system.run_local(one, workers=workers, bytes_per_worker=2 * self._panel_bytes() + 160 * N if local else 0)
-        nk = len(wrt)
-        red = torch.zeros((nk * N + 1,), dtype=torch.float64, device=dev)
-        for slot in accs:
-            for j, k in enumerate(wrt):
-                red[j * N:(j + 1) * N] += accs[slot][k]
-            red[nk * N] += phis[slot][0]
+            _lib.check(lib.hz_misfit(_lib.ptr(d), _lib.ptr(do), d.numel(), float(Wd), _lib.ptr(v), _lib.ptr(phi),
+                                     _lib.current_stream_ptr(dev)))
+            return v
+        red = self._derivative_sweep(wrt, residual, nextra=1)
         parallel.allreduce_sum_(red)
         if not to_host:
             return red
+        nk, N = len(wrt), self.nrow
         host = red.cpu().numpy()
         return float(host[nk * N]), {k: host[j * N:(j + 1) * N].copy() for j, k in enumerate(wrt)}
 
+    # ---- Born modelling, its adjoint and Gauss-Newton products (DESIGN.md §2) ------------------------------------
+    def _dm_to_device(self, dm, wrt, name):
+        import torch
+        self._check_adjoint_supported(name)
+        dev = self._device_ops()['dev']
+        return {k: torch.from_numpy(a).to(dev) for k, a in self._check_dm(dm, wrt).items()}
+
+    def born_dpred(self, dm, wrt=('c',)):
+        """J dm: the exact linearised ("Born") data of a real model perturbation dm = {'c': dc, 'rho': drho} (the
+        keys of ``wrt``, each N float64 values, the layout ``misfit_and_adjoint_gradient`` returns).  Per frequency a
+        forward solve, the tangent of the assembled planes (``hz_assemble_jvp``), the Born secondary source
+        -dA w (``hz_stencil_apply``), an N solve and the receiver extraction.  Returns the (R, S, F) complex128 data,
+        gathered over the frequency shards as ``survey.dpred`` does.  For the viscous problem dc perturbs the real base
+        velocity; where rho is not given (Gardner's rule) density follows dc.  MiniZephyr operators in complex128 only."""
+        wrt = self._check_wrt(wrt)
+        dmd = self._dm_to_device(dm, wrt, 'born_dpred')
+        dd = self._derivative_sweep(wrt, lambda ifreq, uF, dU, extra: self.extract_device(dU), dm=dmd, back=False)
+        return self.survey._gather_freqs(dd).cpu().numpy()
+
+    def born_adjoint(self, v, wrt=('c',)):
+        """J^H v: the exact adjoint of ``born_dpred`` under the real inner products Re sum conj(a) b on data and the
+        dot product on the model, as a dict of N float64 arrays over ``wrt``, all-reduced over the frequency shards.
+        v: (R, S, F) data or the device tensor of ``upload_dobs``.  Per frequency a forward solve, the A^T solve of the
+        back-projected v, ``hz_stencil_xcorr`` and ``hz_assemble_vjp``: the adjoint path of
+        ``misfit_and_adjoint_gradient``, which is born_adjoint(Wd^2 (dpred - dobs))."""
+        import torch
+        wrt = self._check_wrt(wrt)
+        self._check_adjoint_supported('born_adjoint')
+        local = self.system.localFreqIndices
+        v_all = v if isinstance(v, torch.Tensor) else self.upload_dobs(v)
+        red = self._derivative_sweep(wrt, lambda ifreq, uF, dU, extra: v_all[local.index(ifreq)])
+        return self._reduce_model(red, wrt)
+
+    def gauss_newton_hvec(self, dm, Wd=1., wrt=('c',)):
+        """H_GN dm = J^H Wd^2 J dm, the Gauss-Newton Hessian of 0.5 ||Wd (dpred - dobs)||^2 applied to dm, as a dict of
+        N float64 arrays over ``wrt``, with one all-reduce.  Per frequency, all on the device and on one set of
+        factors: the forward solve, the Born solve, the extraction scaled by Wd^2, the A^T solve of its
+        back-projection, ``hz_stencil_xcorr`` and ``hz_assemble_vjp``.  With keepFactors and an unchanged model,
+        nothing is refactored.  Symmetric and positive semi-definite: <dm, H dm> = ||Wd J dm||^2."""
+        wrt = self._check_wrt(wrt)
+        dmd = self._dm_to_device(dm, wrt, 'gauss_newton_hvec')
+        w2 = float(Wd) ** 2
+
+        def weighted(ifreq, uF, dU, extra):
+            return self.extract_device(dU).mul_(w2)
+        red = self._derivative_sweep(wrt, weighted, dm=dmd)
+        return self._reduce_model(red, wrt)
+
+    def _reduce_model(self, red, wrt):
+        parallel.allreduce_sum_(red)
+        N = self.nrow
+        host = red.cpu().numpy()
+        return {k: host[j * N:(j + 1) * N].copy() for j, k in enumerate(wrt)}
 
 class Helm2DProblem(HelmBaseProblem):
     SystemWrapper = MultiFreq
