@@ -225,6 +225,18 @@ int hz_assemble_jvp(hz_handle_t h, const double* dc, const double* drho, const v
 int hz_stencil_apply(const void* dcoef, const void* u, int64_t nx, int64_t nz, int64_t S, double scale_re, double scale_im,
                      void* out, void* stream);
 
+/* Pseudo-Hessian diagonal of MiniZephyr (DESIGN.md §2, "Pseudo-Hessian").  hz_wavefield_lagcorr: the lag correlation of
+ * a forward panel u (complex128, N x S, as the forward solve returns it):  C[l*N + p] = sum_s conj(u[p*S + s]) *
+ * u[(p + delta_l)*S + s] for the 13 lags delta_l = (dz, dx) in the order (0,0), (0,1), (0,2), (1,-2..2), (2,-2..2), zero
+ * where p + delta_l lies outside the grid; C is 13*N complex128, overwritten.
+ * hz_pseudo_hessian: P_m[n] = sum_s ||(d A / d m_n) w_s||^2 (w = conj(u)) of the handle's last hz_assemble, contracted
+ * from C and added into p_c and p_rho (float64, N; either may be NULL, not both).  The c column is
+ * alpha[n] dA/dc_n (alpha complex128, N, may be NULL: 1) plus drho_dc[n] dA/drho_n when drho_dc (float64, N) is given
+ * (Gardner's rule), combined before squaring: the column hz_assemble_jvp applies along e_n.  On the handle's stream;
+ * the same refusals as hz_assemble_vjp.                                                                              */
+int hz_wavefield_lagcorr(const void* u, int64_t nx, int64_t nz, int64_t S, void* C, void* stream);
+int hz_pseudo_hessian(hz_handle_t h, const void* C, const void* alpha, const double* drho_dc, double* p_c, double* p_rho);
+
 /* complex64 variant (hz_create(dtype = HZ_C64)): block inverses are stored in complex64 (planar: a real and an
  * imaginary float32 plane per block) and applied by the tcgen05 tensor cores: kind::tf32 MMAs with 3xTF32 operand
  * splitting (FP32-like products), tiles staged by TMA, accumulators in TMEM, split-K partial sums combined with

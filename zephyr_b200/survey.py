@@ -613,10 +613,11 @@ class HelmBaseProblem(BaseModelDependent):
             out[k] = np.ascontiguousarray(a, dtype=np.float64).ravel()
         return out
 
-    def _derivative_sweep(self, wrt, adjoint_data, dm=None, back=True, nextra=0):
+    def _derivative_sweep(self, wrt, adjoint_data, dm=None, back=True, nextra=0, precond=()):
         """The per-frequency device pipeline of the exact derivatives (DESIGN.md §2).  For every local frequency:
 
-        1. the forward panel uF (``forward_device``);
+        1. the forward panel uF (``forward_device``); if ``precond`` names parameters, the pseudo-Hessian diagonal of
+           each from uF: ``hz_wavefield_lagcorr`` and ``hz_pseudo_hessian`` into per-worker accumulators;
         2. if ``dm`` is given, the Born panel dU = conj(-A^-1 dA w) in a second panel: ``hz_assemble_jvp`` along dm,
            ``hz_stencil_apply`` with scale -1/premul and an N solve over the whole depth range;
         3. v = adjoint_data(ifreq, uF, dU, extra), an (R, S) device tensor (extra: this worker's float64 accumulator
@@ -624,10 +625,10 @@ class HelmBaseProblem(BaseModelDependent):
         4. if ``back``: lambda = A^-T (Rv^H v) (back-projection with the adjoint taps, A^T solve), ``hz_stencil_xcorr``
            of lambda and uF and ``hz_assemble_vjp`` into per-worker accumulators of -Re sum lambda^T (dA/dm) w.
 
-        The caller checks that the operators are supported.  ``dm`` holds float64 device tensors of N over ``wrt``.  Where rho is not given (Gardner's rule), the tangent
-        and the gradient both carry density's dependence on c.  Returns {ifreq: v} if not ``back``; otherwise the
-        float64 device tensor [g_wrt[0] (N), g_wrt[1] (N), ..., extra] summed over the workers of this rank (the
-        caller all-reduces it)."""
+        The caller checks that the operators are supported.  ``dm`` holds float64 device tensors of N over ``wrt``.  Where rho is not given (Gardner's rule), the tangent,
+        the gradient and the c pseudo-Hessian all carry density's dependence on c.  Returns {ifreq: v} if neither
+        ``back`` nor ``precond``; otherwise the float64 device tensor [g_wrt[0] (N), ... (if back), P_precond[0] (N),
+        ..., extra] summed over the workers of this rank (the caller all-reduces it)."""
         import torch
         ops = self._device_ops()
         dev, sv, N = ops['dev'], self.survey, self.nrow
@@ -648,25 +649,34 @@ class HelmBaseProblem(BaseModelDependent):
         taps = {i: self._adjoint_taps(i) for i in local} if back else {}
         alphas = {i: (None if self._adjoint_alpha(i) is None else to_dev(self._adjoint_alpha(i), np.complex128)) for i in local}
         drho_dc = {}
-        if gardner and want_c:
+        if gardner and (want_c or 'c' in precond):
             # rho_f = 310 Re(c_f)^0.25 and Re(c_f) = Re(alpha_f) c  =>  drho_f/dc = rho_f / (4 Re(c))
             cr = np.real(np.asarray(self.systemConfig['c'], dtype=np.complex128)) * np.ones((nz, nx))
             drho_dc = {i: to_dev(0.25 * np.asarray(subs[i].rho, dtype=np.float64).reshape((nz, nx)) / cr, np.float64) for i in local}
-        accs, extras, panels = {}, {}, {}
+        accs, pacc, extras, panels = {}, {}, {}, {}
 
         def one(ifreq, slot):
             stream = _lib.current_stream_ptr(dev)
             if slot not in panels:
                 if back:
                     accs[slot] = {k: torch.zeros((N,), dtype=torch.float64, device=dev) for k in wrt}
+                pacc[slot] = {k: torch.zeros((N,), dtype=torch.float64, device=dev) for k in precond}
                 extras[slot] = torch.zeros((nextra,), dtype=torch.float64, device=dev)
-                panels[slot] = {'uF': None, 'lam': None, 'G': torch.empty((9 * N,), dtype=torch.complex128, device=dev),
+                panels[slot] = {'uF': None, 'lam': None,
+                                'G': torch.empty((9 * N,), dtype=torch.complex128, device=dev) if back or dm is not None else None,
                                 'grho': torch.empty((N,), dtype=torch.float64, device=dev) if rho_scratch else None,
-                                'drho': torch.empty((N,), dtype=torch.float64, device=dev) if tan_rho else None}
+                                'drho': torch.empty((N,), dtype=torch.float64, device=dev) if tan_rho else None,
+                                'C': torch.empty((13 * N,), dtype=torch.complex128, device=dev) if precond else None}
             pn = panels[slot]
             sub = subs[ifreq]
             self._ensure_factors(ifreq, ops['s_z'], evict=workers == 1)
             uF = pn['uF'] = self.forward_device(ifreq, out=pn['uF'])
+            if precond:
+                _lib.check(lib.hz_wavefield_lagcorr(_lib.ptr(uF), nx, nz, sv.nsrc, _lib.ptr(pn['C']), stream))
+                sub._bind_stream()
+                _lib.check(lib.hz_pseudo_hessian(sub.handle, _lib.ptr(pn['C']), _lib.ptr(alphas[ifreq]),
+                                                 _lib.ptr(drho_dc.get(ifreq)) if 'c' in precond else None,
+                                                 _lib.ptr(pacc[slot].get('c')), _lib.ptr(pacc[slot].get('rho'))), sub.handle)
             dU = None
             if dm is not None:
                 dc, drho = dm.get('c'), dm.get('rho')
@@ -694,22 +704,44 @@ class HelmBaseProblem(BaseModelDependent):
                            sub.handle)
                 if want_rho:
                     accs[slot]['rho'] += pn['grho']
-                if drho_dc:
+                if drho_dc and want_c:
                     accs[slot]['c'] += pn['grho'] * drho_dc[ifreq]
             if not self.system.keepFactors:
                 del sub.factors
             return None if back else v
-        per_worker = 2 * self._panel_bytes() + 160 * N + (8 * N if tan_rho else 0)
+        if back or dm is not None:
+            per_worker = 2 * self._panel_bytes() + 160 * N + (8 * N if tan_rho else 0)
+        else:                                                   # pseudo_hessian alone: the forward panel only
+            per_worker = self._panel_bytes()
+        per_worker += (208 + 8 * len(precond)) * N if precond else 0
         res = self.system.run_local(one, workers=workers, bytes_per_worker=per_worker if local else 0)
-        if not back:
+        if not back and not precond:
             return res
-        nk = len(wrt)
+        parts = [(accs, k) for k in (wrt if back else ())] + [(pacc, k) for k in precond]
+        nk = len(parts)
         red = torch.zeros((nk * N + nextra,), dtype=torch.float64, device=dev)
-        for slot in accs:
-            for j, k in enumerate(wrt):
-                red[j * N:(j + 1) * N] += accs[slot][k]
+        for slot in panels:
+            for j, (acc, k) in enumerate(parts):
+                red[j * N:(j + 1) * N] += acc[slot][k]
             red[nk * N:] += extras[slot]
         return red
+
+    def _residual_source(self, dobs, Wd):
+        """The adjoint_data of ``_derivative_sweep`` for the misfit: v = Wd^2 (Rv u - dobs), phi added into extra[0]."""
+        import torch
+        local = self.system.localFreqIndices
+        do_all = dobs if isinstance(dobs, torch.Tensor) else self.upload_dobs(dobs)
+        lib = _lib.get_lib()
+        dev = self._device_ops()['dev']
+
+        def residual(ifreq, uF, dU, phi):
+            d = self.extract_device(uF)
+            do = do_all[local.index(ifreq)]
+            v = torch.empty_like(d)
+            _lib.check(lib.hz_misfit(_lib.ptr(d), _lib.ptr(do), d.numel(), float(Wd), _lib.ptr(v), _lib.ptr(phi),
+                                     _lib.current_stream_ptr(dev)))
+            return v
+        return residual
 
     def misfit_and_adjoint_gradient(self, dobs, Wd=1., wrt=('c',), to_host=True):
         """phi = 0.5 ||Wd (dpred - dobs)||^2 and its exact gradient with respect to the model parameters named in
@@ -723,22 +755,9 @@ class HelmBaseProblem(BaseModelDependent):
         Re(c)^0.25), g_c includes the change of rho with c and g_rho is the partial derivative at fixed c.  dobs: the
         (R, S, F) data or the device tensor from ``upload_dobs``.  to_host=False returns the all-reduced device
         tensor [g_wrt[0] (N), g_wrt[1] (N), ..., phi] (float64) instead.  MiniZephyr operators in complex128 only."""
-        import torch
         wrt = self._check_wrt(wrt)
         self._check_adjoint_supported()
-        local = self.system.localFreqIndices
-        do_all = dobs if isinstance(dobs, torch.Tensor) else self.upload_dobs(dobs)
-        lib = _lib.get_lib()
-        dev = self._device_ops()['dev']
-
-        def residual(ifreq, uF, dU, phi):
-            d = self.extract_device(uF)
-            do = do_all[local.index(ifreq)]
-            v = torch.empty_like(d)
-            _lib.check(lib.hz_misfit(_lib.ptr(d), _lib.ptr(do), d.numel(), float(Wd), _lib.ptr(v), _lib.ptr(phi),
-                                     _lib.current_stream_ptr(dev)))
-            return v
-        red = self._derivative_sweep(wrt, residual, nextra=1)
+        red = self._derivative_sweep(wrt, self._residual_source(dobs, Wd), nextra=1)
         parallel.allreduce_sum_(red)
         if not to_host:
             return red
@@ -793,6 +812,36 @@ class HelmBaseProblem(BaseModelDependent):
             return self.extract_device(dU).mul_(w2)
         red = self._derivative_sweep(wrt, weighted, dm=dmd)
         return self._reduce_model(red, wrt)
+
+    # ---- pseudo-Hessian diagonal (DESIGN.md §2) -------------------------------------------------------------------
+    def pseudo_hessian(self, wrt=('c',)):
+        """The pseudo-Hessian diagonal of Shin, Jang & Min (2001): P_m[n] = sum_f sum_s ||(dA_f/dm_n) w_{f,s}||^2 for
+        each m in ``wrt`` ('c', 'rho'), the energy of the virtual sources of node n.  A diagonal scaling for the
+        exact gradient and for CG on ``gauss_newton_hvec``, or an illumination map; it needs no data.  Per frequency
+        a forward solve, the lag correlation of the forward panel (``hz_wavefield_lagcorr``) and its contraction with
+        the derivative of the assembly (``hz_pseudo_hessian``), all on the device; one all-reduce.  The derivative is
+        the one of the gradient and the Born methods: for the viscous problem with respect to the real base velocity,
+        and where rho is not given (Gardner's rule) the c column includes density's dependence on c.  Returns
+        {name: float64 array of N} over ``wrt``, all >= 0.  MiniZephyr operators in complex128 only."""
+        wrt = self._check_wrt(wrt)
+        self._check_adjoint_supported('pseudo_hessian')
+        red = self._derivative_sweep((), lambda ifreq, uF, dU, extra: None, back=False, precond=wrt)
+        return self._reduce_model(red, wrt)
+
+    def misfit_gradient_and_pseudo_hessian(self, dobs, Wd=1., wrt=('c',)):
+        """``misfit_and_adjoint_gradient`` and ``pseudo_hessian`` in one sweep: the pseudo-Hessian comes from the
+        forward panel the gradient already computes, for two extra kernels per frequency and no extra solve, with one
+        all-reduce of [g..., P..., phi].  This is the call a preconditioned FWI iteration makes.  Returns
+        (phi, {name: g}, {name: P}) over ``wrt``, each as the two methods return them."""
+        wrt = self._check_wrt(wrt)
+        self._check_adjoint_supported('misfit_gradient_and_pseudo_hessian')
+        red = self._derivative_sweep(wrt, self._residual_source(dobs, Wd), nextra=1, precond=wrt)
+        parallel.allreduce_sum_(red)
+        nk, N = len(wrt), self.nrow
+        host = red.cpu().numpy()
+        g = {k: host[j * N:(j + 1) * N].copy() for j, k in enumerate(wrt)}
+        P = {k: host[(nk + j) * N:(nk + j + 1) * N].copy() for j, k in enumerate(wrt)}
+        return float(host[2 * nk * N]), g, P
 
     def _reduce_model(self, red, wrt):
         parallel.allreduce_sum_(red)
