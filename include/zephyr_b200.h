@@ -237,6 +237,22 @@ int hz_stencil_apply(const void* dcoef, const void* u, int64_t nx, int64_t nz, i
 int hz_wavefield_lagcorr(const void* u, int64_t nx, int64_t nz, int64_t S, void* C, void* stream);
 int hz_pseudo_hessian(hz_handle_t h, const void* C, const void* alpha, const double* drho_dc, double* p_c, double* p_rho);
 
+/* Gauss-Newton Hessian diagonal of MiniZephyr, H_nn = sum_r,s |(J e_n)_{r,s}|^2 without the data weight (DESIGN.md §2,
+ * "Gauss-Newton diagonal").  hz_wavefield_lagcorr4: the lag correlation of radius 4 of a panel u (complex128, N x S):
+ * C41[l*N + p] = sum_s conj(u[p*S + s]) * u[(p + delta_l)*S + s] for the 41 lags delta_l = (dz, dx) in the order
+ * (0,0), (0,1..4), (1,-4..4), (2,-4..4), (3,-4..4), (4,-4..4), zero where p + delta_l lies outside the grid; C41 is
+ * 41*N complex128, overwritten.  Its planes of the 13 lags of hz_wavefield_lagcorr hold the same values.
+ * hz_gauss_newton_diag: with C41 from the forward panel u (C(p, p') = sum_s w_s[p] conj(w_s[p']), w = conj(u)) and
+ * Gam13 = hz_wavefield_lagcorr of the conjugated receiver Green's functions conj(g_r), g_r = A^-T conj(Rv[r, .])^T
+ * (Gam(i, i') = sum_r g_r[i] conj(g_r[i'])), adds
+ *     H_m[n] = sum_{i,i'} Gam(i, i') sum_{a,b} (dA/dm_n)[i, i + off(a)] conj((dA/dm_n)[i', i' + off(b)]) C(i + off(a), i' + off(b))
+ * into p_c and p_rho (float64, N; either may be NULL, not both), for the derivative of the handle's last hz_assemble
+ * with alpha and drho_dc as in hz_pseudo_hessian.  With Gam the identity (zero-lag plane 1, the others 0) this is
+ * hz_pseudo_hessian.  On the handle's stream; the same refusals as hz_pseudo_hessian.                                 */
+int hz_wavefield_lagcorr4(const void* u, int64_t nx, int64_t nz, int64_t S, void* C41, void* stream);
+int hz_gauss_newton_diag(hz_handle_t h, const void* C41, const void* Gam13, const void* alpha, const double* drho_dc, double* p_c,
+                         double* p_rho);
+
 /* complex64 variant (hz_create(dtype = HZ_C64)): block inverses are stored in complex64 (planar: a real and an
  * imaginary float32 plane per block) and applied by the tcgen05 tensor cores: kind::tf32 MMAs with 3xTF32 operand
  * splitting (FP32-like products), tiles staged by TMA, accumulators in TMEM, split-K partial sums combined with

@@ -60,6 +60,8 @@ SIGNATURES = {
     'hz_assemble_jvp': (_int, [_vp, _vp, _vp, _vp, _vp]),
     'hz_wavefield_lagcorr': (_int, [_vp, _i64, _i64, _i64, _vp, _vp]),
     'hz_pseudo_hessian': (_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
+    'hz_wavefield_lagcorr4': (_int, [_vp, _i64, _i64, _i64, _vp, _vp]),
+    'hz_gauss_newton_diag': (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     'hz_scatter_coo_c64': (_int, [_vp, _i64, _i64, _vp, _vp, _vp, _f64, _f64, _vp]),
     'hz_spmm_csr_c64': (_int, [_i64, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp, _i64, _i64, _int, _vp]),
     'hz_gradient_c64': (_int, [_vp, _vp, _i64, _i64, _vp, _vp, _vp]),

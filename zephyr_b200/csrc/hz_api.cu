@@ -1100,7 +1100,8 @@ static void preload_factor_kernels() {
     preload_kernel(nearest_index_kernel); preload_kernel(kaiser_taps_kernel);
     preload_kernel(stencil_xcorr_kernel); preload_kernel(assemble_mz_vjp_kernel);
     preload_kernel(stencil_apply_kernel); preload_kernel(assemble_mz_jvp_kernel);
-    preload_kernel(wavefield_lagcorr_kernel); preload_kernel(pseudo_hessian_mz_kernel);
+    preload_kernel(wavefield_lagcorr_kernel<LAGCORR2_ARGS>); preload_kernel(pseudo_hessian_mz_kernel);
+    preload_kernel(wavefield_lagcorr_kernel<LAGCORR4_ARGS>); preload_kernel(gauss_newton_diag_mz_kernel);
     preload_panel_kernels<cplx>();
     preload_panel_kernels<cplxf>();
     zgemm_for_each_instance<0>([](auto kfn) { preload_kernel(kfn); });
@@ -2035,18 +2036,29 @@ int hz_assemble_jvp(hz_handle_t h, const double* dc, const double* drho, const v
     return HZ_OK;
 }
 
-int hz_wavefield_lagcorr(const void* u, int64_t nx, int64_t nz, int64_t S, void* C, void* stream) {
-    if (!u || !C) return fail(nullptr, HZ_EINVAL, "hz_wavefield_lagcorr: NULL argument");
-    if (nx < 3 || nz < 3 || nx > 32768 || nz > (1 << 24) || S < 1) return fail(nullptr, HZ_EINVAL, "hz_wavefield_lagcorr: nx, nz or S out of range");
-    const i64 runs = (nx + LAGCORR_RUN - 1) / LAGCORR_RUN;
-    if (nz * runs > 0x7fffffffLL) return fail(nullptr, HZ_EINVAL, "hz_wavefield_lagcorr: grid too large");
-    // one pass of a CTA covers threads * LAGCORR_SPL sources: size the block so that no lane runs on zeros only
-    const i64 per_lane = (S + LAGCORR_SPL - 1) / LAGCORR_SPL;
-    const int threads = per_lane >= 256 ? 256 : (int)((per_lane + 31) / 32 * 32);
-    HZ_LAUNCH_IND(wavefield_lagcorr_kernel, dim3((unsigned)(nz * runs)), dim3(threads), (size_t)(threads / 32) * LAGCORR_RUN * 32 * sizeof(double),
+// the lag correlation of radius R (hz_precond.cuh): one launcher for both radii
+template <int R, int RUN, int SPL, int MAXT, int MINB>
+static int wavefield_lagcorr_launch(const char* name, const void* u, int64_t nx, int64_t nz, int64_t S, void* C, void* stream) {
+    if (!u || !C) return fail(nullptr, HZ_EINVAL, std::string(name) + ": NULL argument");
+    if (nx < 3 || nz < 3 || nx > 32768 || nz > (1 << 24) || S < 1) return fail(nullptr, HZ_EINVAL, std::string(name) + ": nx, nz or S out of range");
+    const i64 runs = (nx + RUN - 1) / RUN;
+    if (nz * runs > 0x7fffffffLL) return fail(nullptr, HZ_EINVAL, std::string(name) + ": grid too large");
+    // one pass of a CTA covers threads * SPL sources: size the block so that no lane runs on zeros only
+    const i64 per_lane = (S + SPL - 1) / SPL;
+    const int threads = per_lane >= MAXT ? MAXT : (int)((per_lane + 31) / 32 * 32);
+    auto kfn = wavefield_lagcorr_kernel<R, RUN, SPL, MAXT, MINB>;
+    HZ_LAUNCH_IND(kfn, dim3((unsigned)(nz * runs)), dim3(threads), (size_t)(threads / 32) * RUN * LagShape<R>::chunks * 32 * sizeof(double),
                   (cudaStream_t)stream, (const cplx*)u, (int)nx, (int)nz, (i64)S, (cplx*)C);
     HZ_CHECK_LAUNCH(nullptr);
     return HZ_OK;
+}
+
+int hz_wavefield_lagcorr(const void* u, int64_t nx, int64_t nz, int64_t S, void* C, void* stream) {
+    return wavefield_lagcorr_launch<LAGCORR2_ARGS>("hz_wavefield_lagcorr", u, nx, nz, S, C, stream);
+}
+
+int hz_wavefield_lagcorr4(const void* u, int64_t nx, int64_t nz, int64_t S, void* C, void* stream) {
+    return wavefield_lagcorr_launch<LAGCORR4_ARGS>("hz_wavefield_lagcorr4", u, nx, nz, S, C, stream);
 }
 
 int hz_pseudo_hessian(hz_handle_t h, const void* C, const void* alpha, const double* drho_dc, double* p_c, double* p_rho) {
@@ -2060,6 +2072,24 @@ int hz_pseudo_hessian(hz_handle_t h, const void* C, const void* alpha, const dou
     const int threads = 128;
     HZ_LAUNCH_EW(pseudo_hessian_mz_kernel, dim3((unsigned)((h->N + threads - 1) / threads)), dim3(threads), 0, h->stream, (const cplx*)h->c,
                  (const cplx*)h->Kp, (const double*)h->binv, (const cplx*)C, (const cplx*)alpha, drho_dc, h->asm_p, p_c, p_rho);
+    HZ_CHECK_LAUNCH(h);
+    return HZ_OK;
+}
+
+int hz_gauss_newton_diag(hz_handle_t h, const void* C41, const void* Gam13, const void* alpha, const double* drho_dc, double* p_c,
+                         double* p_rho) {
+    if (!h) return fail(h, HZ_EINVAL, "hz_gauss_newton_diag: NULL handle");
+    if (h->disc != HZ_DISC_MINIZEPHYR || h->dtype != HZ_C128)
+        return fail(h, HZ_ENOTIMPL, "hz_gauss_newton_diag: built for complex128 MiniZephyr handles only");
+    if (!C41 || !Gam13 || (!p_c && !p_rho))
+        return fail(h, HZ_EINVAL, "hz_gauss_newton_diag: C41, Gam13 and at least one of p_c, p_rho are required");
+    if (!h->assembled || !h->asm_from_model)
+        return fail(h, HZ_ESTATE, "hz_gauss_newton_diag: the coefficients must come from hz_assemble of the current model");
+    HZ_CUDA(h, cudaSetDevice(h->device));
+    const int threads = 128;
+    HZ_LAUNCH_EW(gauss_newton_diag_mz_kernel, dim3((unsigned)((h->N + threads - 1) / threads)), dim3(threads), 0, h->stream,
+                 (const cplx*)h->c, (const cplx*)h->Kp, (const double*)h->binv, (const cplx*)C41, (const cplx*)Gam13,
+                 (const cplx*)alpha, drho_dc, h->asm_p, p_c, p_rho);
     HZ_CHECK_LAUNCH(h);
     return HZ_OK;
 }

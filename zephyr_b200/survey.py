@@ -594,6 +594,20 @@ class HelmBaseProblem(BaseModelDependent):
         pm = complex(self.system.subProblems[ifreq].premul)
         return ops[key + '_conj'] if pm == 1 else ops[key + '_conj'] / pm
 
+    def _green_rhs(self, ifreq):
+        """The right-hand sides of the receiver Green's functions of one frequency as COO (row = node, col = receiver,
+        val): column r holds conj(Rv[r, .]) / premul, so that the premultiplied, conjugating A^T solve returns
+        conj(g_r) with g_r = A^-T conj(Rv[r, .])^T.  'fixed' geometry only.  Formed on the caller's stream."""
+        import torch
+        ops = self._device_ops()
+        if 'g_row' not in ops:
+            Rv = self.survey.rVec().tocoo()                                  # (R, N)
+            ops['g_row'] = torch.from_numpy(np.ascontiguousarray(Rv.col, dtype=np.int64)).to(ops['dev'])
+            ops['g_col'] = torch.from_numpy(np.ascontiguousarray(Rv.row, dtype=np.int64)).to(ops['dev'])
+            ops['g_val'] = torch.from_numpy(np.ascontiguousarray(np.conj(Rv.data), dtype=np.complex128)).to(ops['dev'])
+        pm = complex(self.system.subProblems[ifreq].premul)
+        return ops['g_row'], ops['g_col'], (ops['g_val'] if pm == 1 else ops['g_val'] / pm)
+
     @staticmethod
     def _check_wrt(wrt):
         wrt = tuple(wrt)
@@ -613,11 +627,14 @@ class HelmBaseProblem(BaseModelDependent):
             out[k] = np.ascontiguousarray(a, dtype=np.float64).ravel()
         return out
 
-    def _derivative_sweep(self, wrt, adjoint_data, dm=None, back=True, nextra=0, precond=()):
+    def _derivative_sweep(self, wrt, adjoint_data, dm=None, back=True, nextra=0, precond=(), gndiag=()):
         """The per-frequency device pipeline of the exact derivatives (DESIGN.md §2).  For every local frequency:
 
         1. the forward panel uF (``forward_device``); if ``precond`` names parameters, the pseudo-Hessian diagonal of
-           each from uF: ``hz_wavefield_lagcorr`` and ``hz_pseudo_hessian`` into per-worker accumulators;
+           each from uF: ``hz_wavefield_lagcorr`` and ``hz_pseudo_hessian`` into per-worker accumulators; if ``gndiag``
+           names parameters, the Gauss-Newton diagonal of each without Wd^2: the receiver Green's functions conj(g_r)
+           (an R-column panel of conjugated taps / premul, a conjugating A^T solve), ``hz_wavefield_lagcorr`` of it,
+           ``hz_wavefield_lagcorr4`` of uF and ``hz_gauss_newton_diag`` into per-worker accumulators ('fixed' only);
         2. if ``dm`` is given, the Born panel dU = conj(-A^-1 dA w) in a second panel: ``hz_assemble_jvp`` along dm,
            ``hz_stencil_apply`` with scale -1/premul and an N solve over the whole depth range;
         3. v = adjoint_data(ifreq, uF, dU, extra), an (R, S) device tensor (extra: this worker's float64 accumulator
@@ -626,9 +643,10 @@ class HelmBaseProblem(BaseModelDependent):
            of lambda and uF and ``hz_assemble_vjp`` into per-worker accumulators of -Re sum lambda^T (dA/dm) w.
 
         The caller checks that the operators are supported.  ``dm`` holds float64 device tensors of N over ``wrt``.  Where rho is not given (Gardner's rule), the tangent,
-        the gradient and the c pseudo-Hessian all carry density's dependence on c.  Returns {ifreq: v} if neither
-        ``back`` nor ``precond``; otherwise the float64 device tensor [g_wrt[0] (N), ... (if back), P_precond[0] (N),
-        ..., extra] summed over the workers of this rank (the caller all-reduces it)."""
+        the gradient and the c pseudo-Hessian and Gauss-Newton diagonal all carry density's dependence on c.  Returns
+        {ifreq: v} if none of ``back``, ``precond``, ``gndiag``; otherwise the float64 device tensor [g_wrt[0] (N), ...
+        (if back), P_precond[0] (N), ..., H_gndiag[0] (N), ..., extra] summed over the workers of this rank (the caller
+        all-reduces it)."""
         import torch
         ops = self._device_ops()
         dev, sv, N = ops['dev'], self.survey, self.nrow
@@ -649,11 +667,13 @@ class HelmBaseProblem(BaseModelDependent):
         taps = {i: self._adjoint_taps(i) for i in local} if back else {}
         alphas = {i: (None if self._adjoint_alpha(i) is None else to_dev(self._adjoint_alpha(i), np.complex128)) for i in local}
         drho_dc = {}
-        if gardner and (want_c or 'c' in precond):
+        if gardner and (want_c or 'c' in precond or 'c' in gndiag):
             # rho_f = 310 Re(c_f)^0.25 and Re(c_f) = Re(alpha_f) c  =>  drho_f/dc = rho_f / (4 Re(c))
             cr = np.real(np.asarray(self.systemConfig['c'], dtype=np.complex128)) * np.ones((nz, nx))
             drho_dc = {i: to_dev(0.25 * np.asarray(subs[i].rho, dtype=np.float64).reshape((nz, nx)) / cr, np.float64) for i in local}
-        accs, pacc, extras, panels = {}, {}, {}, {}
+        green = {i: self._green_rhs(i) for i in local} if gndiag else {}
+        R = sv.nrec
+        accs, pacc, hacc, extras, panels = {}, {}, {}, {}, {}
 
         def one(ifreq, slot):
             stream = _lib.current_stream_ptr(dev)
@@ -661,12 +681,15 @@ class HelmBaseProblem(BaseModelDependent):
                 if back:
                     accs[slot] = {k: torch.zeros((N,), dtype=torch.float64, device=dev) for k in wrt}
                 pacc[slot] = {k: torch.zeros((N,), dtype=torch.float64, device=dev) for k in precond}
+                hacc[slot] = {k: torch.zeros((N,), dtype=torch.float64, device=dev) for k in gndiag}
                 extras[slot] = torch.zeros((nextra,), dtype=torch.float64, device=dev)
                 panels[slot] = {'uF': None, 'lam': None,
                                 'G': torch.empty((9 * N,), dtype=torch.complex128, device=dev) if back or dm is not None else None,
                                 'grho': torch.empty((N,), dtype=torch.float64, device=dev) if rho_scratch else None,
                                 'drho': torch.empty((N,), dtype=torch.float64, device=dev) if tan_rho else None,
-                                'C': torch.empty((13 * N,), dtype=torch.complex128, device=dev) if precond else None}
+                                'C': torch.empty((13 * N,), dtype=torch.complex128, device=dev) if precond or gndiag else None,
+                                'Gr': torch.empty((N, R), dtype=torch.complex128, device=dev) if gndiag else None,
+                                'C41': torch.empty((41 * N,), dtype=torch.complex128, device=dev) if gndiag else None}
             pn = panels[slot]
             sub = subs[ifreq]
             self._ensure_factors(ifreq, ops['s_z'], evict=workers == 1)
@@ -677,6 +700,19 @@ class HelmBaseProblem(BaseModelDependent):
                 _lib.check(lib.hz_pseudo_hessian(sub.handle, _lib.ptr(pn['C']), _lib.ptr(alphas[ifreq]),
                                                  _lib.ptr(drho_dc.get(ifreq)) if 'c' in precond else None,
                                                  _lib.ptr(pacc[slot].get('c')), _lib.ptr(pacc[slot].get('rho'))), sub.handle)
+            if gndiag:
+                # conj(g_r) = conj(A^-T conj(Rv[r, .])^T): the premultiplied, conjugating A^T solve of taps / premul
+                Gr = pn['Gr']
+                Gr.zero_()
+                row, col, val = green[ifreq]
+                _lib.check(lib.hz_scatter_coo(_lib.ptr(Gr), R, row.numel(), _lib.ptr(row), _lib.ptr(col), _lib.ptr(val), 1., 0., stream))
+                sub.solve_device(Gr, ops['b_z'], conjugate=True, trans='T')
+                _lib.check(lib.hz_wavefield_lagcorr(_lib.ptr(Gr), nx, nz, R, _lib.ptr(pn['C']), stream))
+                _lib.check(lib.hz_wavefield_lagcorr4(_lib.ptr(uF), nx, nz, sv.nsrc, _lib.ptr(pn['C41']), stream))
+                sub._bind_stream()
+                _lib.check(lib.hz_gauss_newton_diag(sub.handle, _lib.ptr(pn['C41']), _lib.ptr(pn['C']), _lib.ptr(alphas[ifreq]),
+                                                    _lib.ptr(drho_dc.get(ifreq)) if 'c' in gndiag else None,
+                                                    _lib.ptr(hacc[slot].get('c')), _lib.ptr(hacc[slot].get('rho'))), sub.handle)
             dU = None
             if dm is not None:
                 dc, drho = dm.get('c'), dm.get('rho')
@@ -711,13 +747,14 @@ class HelmBaseProblem(BaseModelDependent):
             return None if back else v
         if back or dm is not None:
             per_worker = 2 * self._panel_bytes() + 160 * N + (8 * N if tan_rho else 0)
-        else:                                                   # pseudo_hessian alone: the forward panel only
+        else:                                                   # pseudo_hessian / gauss_newton_diagonal alone: the forward panel
             per_worker = self._panel_bytes()
         per_worker += (208 + 8 * len(precond)) * N if precond else 0
+        per_worker += (N * R * 16 + (656 + (0 if precond else 208) + 8 * len(gndiag)) * N) if gndiag else 0
         res = self.system.run_local(one, workers=workers, bytes_per_worker=per_worker if local else 0)
-        if not back and not precond:
+        if not back and not precond and not gndiag:
             return res
-        parts = [(accs, k) for k in (wrt if back else ())] + [(pacc, k) for k in precond]
+        parts = [(accs, k) for k in (wrt if back else ())] + [(pacc, k) for k in precond] + [(hacc, k) for k in gndiag]
         nk = len(parts)
         red = torch.zeros((nk * N + nextra,), dtype=torch.float64, device=dev)
         for slot in panels:
@@ -842,6 +879,44 @@ class HelmBaseProblem(BaseModelDependent):
         g = {k: host[j * N:(j + 1) * N].copy() for j, k in enumerate(wrt)}
         P = {k: host[(nk + j) * N:(nk + j + 1) * N].copy() for j, k in enumerate(wrt)}
         return float(host[2 * nk * N]), g, P
+
+    # ---- Gauss-Newton Hessian diagonal (DESIGN.md §2) -------------------------------------------------------------
+    def _check_gauss_newton_diagonal_supported(self, name):
+        self._check_adjoint_supported(name)
+        if self.survey.mode != 'fixed':
+            raise NotImplementedError("%s needs 'fixed' receivers: with 'relative' geometry the receiver Green's functions "
+                                      "would be one per (receiver, source) pair" % name)
+
+    def gauss_newton_diagonal(self, Wd=1., wrt=('c',)):
+        """The exact diagonal of the Gauss-Newton Hessian J^H Wd^2 J (Pratt, Shin & Hicks 1998):
+        H_m[n] = Wd^2 sum_f sum_s sum_r |(J e_n)_{r,s,f}|^2 for each m in ``wrt`` ('c', 'rho'), the diagonal of
+        ``gauss_newton_hvec``.  Unlike ``pseudo_hessian`` it accounts for where the receivers are.  Per frequency, all
+        on the device: the forward solve, one A^T solve of the R receiver columns (the receiver Green's functions), the
+        lag correlations of both panels (``hz_wavefield_lagcorr``, ``hz_wavefield_lagcorr4``) and their contraction
+        with the derivative of the assembly (``hz_gauss_newton_diag``); the cost has no S x R term.  One all-reduce.
+        The derivative is the one of the gradient and the Born methods (viscous: real base velocity; Gardner's rule:
+        the c column includes density's dependence on c).  Returns {name: float64 array of N} over ``wrt``, >= 0 up to
+        rounding.  MiniZephyr operators in complex128 with 'fixed' receivers only."""
+        wrt = self._check_wrt(wrt)
+        self._check_gauss_newton_diagonal_supported('gauss_newton_diagonal')
+        red = self._derivative_sweep((), lambda ifreq, uF, dU, extra: None, back=False, gndiag=wrt)
+        red.mul_(float(Wd) ** 2)
+        return self._reduce_model(red, wrt)
+
+    def misfit_gradient_and_gauss_newton_diagonal(self, dobs, Wd=1., wrt=('c',)):
+        """``misfit_and_adjoint_gradient`` and ``gauss_newton_diagonal`` in one sweep: the diagonal reuses the forward
+        panel of the gradient, so it adds one R-column A^T solve and three kernels per frequency, with one all-reduce of
+        [g..., H..., phi].  Returns (phi, {name: g}, {name: H}) over ``wrt``, each as the two methods return them."""
+        wrt = self._check_wrt(wrt)
+        self._check_gauss_newton_diagonal_supported('misfit_gradient_and_gauss_newton_diagonal')
+        red = self._derivative_sweep(wrt, self._residual_source(dobs, Wd), nextra=1, gndiag=wrt)
+        nk, N = len(wrt), self.nrow
+        red[nk * N:2 * nk * N].mul_(float(Wd) ** 2)
+        parallel.allreduce_sum_(red)
+        host = red.cpu().numpy()
+        g = {k: host[j * N:(j + 1) * N].copy() for j, k in enumerate(wrt)}
+        H = {k: host[(nk + j) * N:(nk + j + 1) * N].copy() for j, k in enumerate(wrt)}
+        return float(host[2 * nk * N]), g, H
 
     def _reduce_model(self, red, wrt):
         parallel.allreduce_sum_(red)
